@@ -3,6 +3,8 @@
 
   python bench.py --gpus N --steps K --warmup W [--config 2|3|4|5]   our arm (one process per GPU under torchrun)
   python bench.py --impl reference --gpus N ... [--config ...]       the restated reference CPU path (oracle/) on host cores
+  python bench.py ... --dump-outputs DIR                             also writes the outputs of the last timed step (see
+                                                                     dump_outputs) for an output-for-output comparison
 
 BASELINE.json configs (SURVEY.md §8):
   2 (default, the headline line)  training step, 6 enc/dec pairs, d 256, 8 heads, 100 queries, 20x20 features, 16 images
@@ -107,6 +109,29 @@ def algorithmic_flops_per_step(cfg, B, C, A, training=True):
 def cost_algorithmic_bytes(B, T, Q, C, A):
     """SURVEY.md §8d: every input read once, the cost matrix written once (fp32)."""
     return 4.0 * B * (Q * C + Q * A + 4 * Q + T * C + T * A + 4 * T + T * Q)
+
+
+DUMP_MAX_ELEMENTS = 1 << 22         # per array; a larger one is reduced to a fixed, seeded sample of its elements
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(outputs, out_dir):
+    """`--dump-outputs`: writes each output as `out_dir/<name>.npy` (float32, or float64 for integer arrays) so that two
+    builds run with the same arguments can be compared output for output.  An array of more than DUMP_MAX_ELEMENTS is
+    flattened and reduced to the elements at sorted indices drawn with seed 0, which depend only on its size."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype.kind == "f" and a.dtype.itemsize <= 4 else np.float64)
+        if a.size > DUMP_MAX_ELEMENTS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))]
+        arrays[name] = a
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_MAX_BYTES}-byte limit")
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -406,13 +431,15 @@ class Ctx:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    def timed_device(self, step, steps):
-        """EXACTLY `steps` steps, each bracketed by CUDA events on the launching stream with an L2 flush (256 MiB write)
-        outside the brackets; barrier + synchronize on both sides; max over ranks of the summed time."""
+    def timed_device(self, step, steps, reset=None):
+        """EXACTLY `steps` steps, each bracketed by CUDA events on the launching stream with `reset()` (when given) and an
+        L2 flush (256 MiB write) outside the brackets; barrier + synchronize on both sides; max over ranks of the summed time."""
         import torch
         times = []
         self.barrier()
         for _ in range(steps):
+            if reset is not None:
+                reset()
             self.flush.zero_()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record(); step(); b.record()
@@ -433,7 +460,8 @@ class Ctx:
         return self.max_over_ranks(time.perf_counter() - t0) / steps, out
 
 
-def run_train(cx, cfg_id, cfg):
+def run_train(cx, cfg_id, cfg, outputs=None):
+    """`outputs` (optional dict): receives what the last timed step computed, as host arrays."""
     import torch
     from boosted_detr_b200 import _lib
     from boosted_detr_b200.graph import GraphedTrainStep
@@ -443,6 +471,18 @@ def run_train(cx, cfg_id, cfg):
     B, C, A = per_gpu_batch(cfg, world), cfg["C"], cfg["A"]
     model = make_model(cfg, cfg_id=cfg_id)
     DataParallel(model, overlap=not args.no_overlap)
+    # The state a step updates in place: the weights, the BatchNorm moving statistics and the optimizer's momentum (zero
+    # before the first update).  The split-K weight gradients accumulate with float reduce-adds, so consecutive steps
+    # drift apart from run to run; restoring the initial state before every device-timed step makes each of them --
+    # and the last one, whose outputs --dump-outputs writes -- compute the same thing from the same inputs in every run.
+    in_place = [model._flat[0]] + [o._weights[k] for _, o, k in model.named_weights() if k in o._non_trainable]
+    initial = [t.clone() for t in in_place]
+
+    def reset():
+        for t, t0 in zip(in_place, initial):
+            t.copy_(t0)
+        if model.optimizer._accum is not None:
+            model.optimizer._accum.zero_()
     batch = synth_batch(rank, B, C, A, cfg)
     if args.no_graph:
         dev_batch = {k: torch.from_numpy(v).cuda() for k, v in batch.items()}
@@ -452,7 +492,6 @@ def run_train(cx, cfg_id, cfg):
         step = gs.replay
     for _ in range(max(args.warmup, 3)):
         step()
-    sec = cx.timed_device(step, args.steps)
     # ---- end-to-end: public API with HOST buffers (pinned H2D in, metric means + matcher status D2H out) every step.
     # The next batch's H2D copy is queued right behind the running step's launch (GraphedTrainStep prefetch).
     host_batch = {k: torch.from_numpy(np.ascontiguousarray(v, np.int32 if k == "num_objects" else np.float32)).pin_memory()
@@ -472,6 +511,15 @@ def run_train(cx, cfg_id, cfg):
     else:
         e2e_fn = lambda: gs(host_batch)
     e2e_sec, logs = cx.timed_e2e(e2e_fn, args.steps)
+    # ---- device arm (the headline): inputs resident in HBM, each step from the initial state (reset outside the brackets)
+    sec = cx.timed_device(step, args.steps, reset)
+    if outputs is not None:
+        # what a caller of the step holds after it: the metric tensors and the updated variables (by variable name, so
+        # that the layout of the flat buffer does not enter the comparison)
+        outputs.update({k: v.float().cpu().numpy() for k, v in model.metric_tensors.items()})
+        outputs["metric_means"] = model.metric_means.cpu().numpy()
+        w = model.get_weights_dict()
+        outputs["weights"] = np.concatenate([w[n].reshape(-1) for n in sorted(w)])
     h2d = sum(v.nbytes for v in batch.values())
     d2h = 4 * 6 + 4 * cfg["N"] * B                         # six metric means + per-block, per-image matcher status flags
     launches = None
@@ -499,9 +547,10 @@ def count_launches(model, batch):
     return int(lib.bdetr_launch_count())
 
 
-def run_matcher(cx, cfg):
+def run_matcher(cx, cfg, outputs=None):
     """Config 4.  Device arm: inputs resident in HBM.  e2e arm: MatchingLoss public call on pinned HOST arrays (H2D of
-    targets + predictions, D2H of the [5,B] losses, the [B,T] assignment and the status flags)."""
+    targets + predictions, D2H of the [5,B] losses, the [B,T] assignment and the status flags).  `outputs` as in
+    run_train."""
     import torch
     from boosted_detr_b200 import _lib
     from boosted_detr_b200.device import ptr, stream_ptr
@@ -548,6 +597,8 @@ def run_matcher(cx, cfg):
         raise_for_status(h_out[2])
         return h_out[0]
     e2e_sec, _ = cx.timed_e2e(e2e, cx.args.steps)
+    if outputs is not None:
+        outputs.update(losses=h_out[0].numpy().copy(), assignment=h_out[1].numpy().astype(np.float64), iou=iou.cpu().numpy())
     # the pieces, each alone (graph of 20 back-to-back launches, L2 flushed)
     s = stream_ptr
     parts = {
@@ -565,9 +616,9 @@ def run_matcher(cx, cfg):
                     "ms_per_step": e2e_sec * 1e3, "us_per_image": e2e_sec / B * 1e6}}
 
 
-def run_infer(cx, cfg, also_faithful=True):
+def run_infer(cx, cfg, also_faithful=True, outputs=None):
     """Config 5: inference only.  Device arm: features resident in HBM; e2e arm: `model(inputs)` on pinned host features
-    (H2D every step) + D2H of the three prediction tensors."""
+    (H2D every step) + D2H of the three prediction tensors.  `outputs` as in run_train (the full-size variant)."""
     import torch
     from boosted_detr_b200 import _lib
     lib = _lib.load()
@@ -588,7 +639,7 @@ def run_infer(cx, cfg, also_faithful=True):
         torch.cuda.synchronize()
         launches = int(lib.bdetr_launch_count())
         assert all(bool(torch.isfinite(t).all()) for t in preds)
-        steps = max(3, min(cx.args.steps, 10))
+        steps = cx.args.steps
         sec = cx.timed_device(fn, steps)
         hp = [torch.empty(t.shape).pin_memory() for t in preds]
 
@@ -598,7 +649,9 @@ def run_infer(cx, cfg, also_faithful=True):
                 h.copy_(t, non_blocking=True)
             torch.cuda.current_stream().synchronize()
             return hp
-        e2e_sec, _ = cx.timed_e2e(e2e, steps)
+        e2e_sec, last = cx.timed_e2e(e2e, steps)
+        if outputs is not None and not tag:
+            outputs.update({k: h.numpy().copy() for k, h in zip(("category", "attribute", "bbox"), last)})
         flops = algorithmic_flops_per_step(c, B, c["C"], c["A"], training=False)
         r = {"value": B * cx.world / sec, "ms_per_step": sec * 1e3, "per_gpu_batch": B, "global_batch": B * cx.world, "steps": steps,
              "tokens": c["rows"] * c["cols"], "algorithmic_tflops": flops / sec / 1e12, "launches_per_step": launches,
@@ -644,7 +697,13 @@ def main():
     ap.add_argument("--no-pdl", action="store_true", help="disable programmatic dependent launch (A/B timing)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--max-seconds", type=float, default=540.0, help="hard wall-clock limit: a wedged run prints what it has and exits")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step as DIR/<name>.npy "
+                    "(rank 0; --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     cfg_id, cfg = args.config, CONFIGS[args.config]
@@ -687,12 +746,15 @@ def main():
         sampler.start()
 
     model = batch = None
+    outputs = {} if args.dump_outputs and rank == 0 else None
     if cfg["kind"] == "train":
-        main_res, model, batch = run_train(cx, cfg_id, cfg)
+        main_res, model, batch = run_train(cx, cfg_id, cfg, outputs)
     elif cfg["kind"] == "matcher":
-        main_res = run_matcher(cx, cfg)
+        main_res = run_matcher(cx, cfg, outputs)
     else:
-        main_res = run_infer(cx, cfg)
+        main_res = run_infer(cx, cfg, outputs=outputs)
+    if outputs is not None:
+        dump_outputs(outputs, args.dump_outputs)
     sampler.stop_flag = True
     line = None
     if rank == 0:
@@ -798,7 +860,6 @@ def main():
             line["cpu_baseline"] = {"error": f"{type(e).__name__}: {e}"[:300]}
     print(json.dumps(line))
     sys.stdout.flush()
-    os._exit(0)
 
 
 if __name__ == "__main__":
