@@ -53,6 +53,13 @@ int proj_group_dgrad(int M, int D, int n, const float *const *dY, const float *c
 
 inline bool tc_rows_ok(long long M) { return M >= 1; }
 
+// The fold's pos / pos_tc / d_pos have L = Lk rows (include/bdetr.h).  The residual reads pos[row % Lq] and the q path's
+// positional gradient runs over Lq rows, so resid_pos and tab_q need Lq == Lk.
+inline bool fold_rows_ok(const bdetr_pos_fold *fold, int Lq, int Lk)
+{
+    return !fold || Lq == Lk || !(fold->resid_pos || fold->tab_q);
+}
+
 }  // namespace
 
 API int bdetr_pos_projection(int L, int D, const float *pos_tc, int n, const float *const *W, const float *const *b,
@@ -82,6 +89,7 @@ API int bdetr_attention_fused_fwd(int B, int Lq, int Lk, int D, int H, const flo
     const float *tab_q = fold ? fold->tab_q : nullptr, *tab_k = fold ? fold->tab_k : nullptr;
     const float *rpos = (fold && fold->resid_pos) ? fold->pos : nullptr;
     BDETR_REQUIRE(!(fold && fold->resid_pos) || fold->pos, BDETR_E_NULL, "resid_pos needs the positional table");
+    BDETR_REQUIRE(fold_rows_ok(fold, Lq, Lk), BDETR_E_BAD_SHAPE, "resid_pos / tab_q need Lq == Lk (pos has Lk rows)");
     const bool self = memory == query && Lq == Lk;
     if (self) {
         const Proj p[3] = {{w->wq, w->bq, sv->qp}, {w->wk, w->bk, sv->kp}, {w->wv, w->bv, sv->vp}};
@@ -126,6 +134,7 @@ API int bdetr_attention_fused_bwd(int B, int Lq, int Lk, int D, int H, const flo
     const bool resid_pos = fold && fold->resid_pos;
     const float *pos_tc = fold ? (fold->pos_tc ? fold->pos_tc : fold->pos) : nullptr;
     const bool want_pos = d_pos != nullptr && (tab_q || tab_k || resid_pos);
+    BDETR_REQUIRE(fold_rows_ok(fold, Lq, Lk), BDETR_E_BAD_SHAPE, "resid_pos / tab_q need Lq == Lk (pos has Lk rows)");
     BDETR_REQUIRE(!want_pos || (sums && pos_tc), BDETR_E_NULL, "positional gradients need `sums` and the positional table");
     const bool need_dq = d_query != nullptr, need_dm = !self && d_memory != nullptr;
     // LayerNorm + residual + dropout; the residual gradient lands in d_resid, the output projection's bias gradient is

@@ -326,7 +326,7 @@ int bdetr_pos_projection(int L, int D, const float *pos_tc, int n, const float *
                          float *const *tab, void *stream);
 
 typedef struct {
-    const float *pos;     /* [L,D] positional table (L = Lk; = Lq too when resid_pos / tab_q are used); NULL: none     */
+    const float *pos;     /* [L,D] positional table (L = Lk; = Lq too when resid_pos / tab_q are used, else BDETR_E_BAD_SHAPE); NULL: none */
     const float *tab_q;   /* [Lq,D] pos Wq + bq, or NULL: q = query Wq + bq                                         */
     const float *tab_k;   /* [Lk,D] pos Wk + bk, or NULL: k = key Wk + bk                                           */
     int resid_pos;        /* 1: the residual is query + pos (encoder, quirk Q4: transformers.py:148 with :226)      */

@@ -49,8 +49,8 @@ def test_config2_size_tf32_vs_fp64_oracle(tc_mode):
     ctx = model.last_ctx_train
     masks = _masks_from_ctx(ctx, B, T, Q)
     tg = (inputs["category"], inputs["attribute"], inputs["bbox"], inputs["num_objects"])
-    out, grads, _ = R.train_step_reference(w, inputs["features"], tg, N, 8, torch.float64, dropout_seed=2024,
-                                           weights=R.model_weights(1.0), forced_masks=masks)
+    out, grads, stats = R.train_step_reference(w, inputs["features"], tg, N, 8, torch.float64, dropout_seed=2024,
+                                               weights=R.model_weights(1.0), forced_masks=masks)
     free, _, _ = R.train_step_reference(w, inputs["features"], tg, N, 8, torch.float64, dropout_seed=2024,
                                         weights=R.model_weights(1.0))
     flips = sum(int((a.numpy() != b.numpy()).any(axis=(1, 2)).sum()) for a, b in zip(free["masks"], masks))
@@ -74,6 +74,15 @@ def test_config2_size_tf32_vs_fp64_oracle(tc_mode):
     rel = (num / den) ** 0.5
     print(f"  whole-gradient relative L2 error {rel:.2e}")
     assert rel < 5e-2
+    # BatchNorm moving statistics (fused heads: per-128-row partials): the increment over momentum * old value, i.e.
+    # the batch statistic's share, so that the exact momentum term does not hide it
+    after = model.get_weights_dict()
+    assert stats
+    e_stats = {k: nerr(after[k] - R.BN_MOMENTUM * w[k].astype(np.float64), ref - R.BN_MOMENTUM * w[k].astype(np.float64))
+               for k, ref in stats.items()}
+    k_worst = max(e_stats, key=e_stats.get)
+    print(f"  BatchNorm moving statistics: worst {k_worst} {e_stats[k_worst]:.2e} over {len(stats)} tensors")
+    assert e_stats[k_worst] < 2e-3, k_worst         # measured 4.4e-4 (B200)
 
 
 def _snapshot(model):
@@ -293,29 +302,69 @@ def test_attention_core_at_config5_length(tc_mode):
 
 def test_frozen_head_batchnorm_runs_in_inference_mode():
     """Keras: BatchNormalization of a frozen layer (trainable = False, reference notebook cell 30) uses its moving
-    statistics and does not update them, even inside a training step; the oracle is told the same."""
+    statistics and does not update them, even inside a training step; the oracle is told the same.  fp32 layer path
+    (B*Q = 24 rows)."""
+    _check_frozen_block0(tc=False)
+
+
+def test_frozen_head_batchnorm_runs_in_inference_mode_fused(tc_mode):
+    """The same on the tf32 fused path (B*Q = 200 rows), where frozen heads run with bn_training 0 / gw NULL and frozen
+    blocks with gw / d_pos NULL: their gradient buffers stay zero."""
+    _check_frozen_block0(tc=True)
+
+
+def _check_frozen_block0(tc):
+    """Block 0 frozen, one training step against the oracle told the same: frozen heads keep their moving statistics,
+    no frozen variable is updated, block 1 and the shared queries match the oracle's gradients."""
     from oracle import reference_path as R
     N = 2
-    model, w, inputs = _model_and_data(N=N, B=2, rows=5, cols=5, Q=12, T=5)
+    if tc:
+        # attribute weight 0: with the attribute term the gradient is ill-conditioned next to the .999 clip and a
+        # tf32-sized perturbation moves it by O(1) (test_model_train_step_tf32)
+        model, w, inputs = _model_and_data(N=N, B=2, rows=20, cols=20, Q=100, T=20, attribute_weight=0.0)
+    else:
+        model, w, inputs = _model_and_data(N=N, B=2, rows=5, cols=5, Q=12, T=5)
     for lst in (model.EncoderTransformerBlocks, model.DecoderBlocks, model.CategoryBlocks, model.AttributeBlocks, model.BoxBlocks):
         lst[0].trainable = False
     model.dropout_seed = None
     model.train_step(inputs)
     torch.cuda.synchronize()
+    assert model._use_fused(torch.empty(inputs["features"].shape)) == tc
     tg = (inputs["category"], inputs["attribute"], inputs["bbox"], inputs["num_objects"])
-    out, grads, stats = R.train_step_reference(w, inputs["features"], tg, N, 8, torch.float64, weights=R.model_weights(1.0),
-                                               frozen_blocks=(0,))
+    B, T, Q = inputs["category"].shape[0], inputs["category"].shape[1], model.num_object_preds
+    masks = _masks_from_ctx(model.last_ctx_train, B, T, Q) if tc else None     # same assignment as the GPU (tf32 near-ties)
+    out, grads, stats = R.train_step_reference(w, inputs["features"], tg, N, 8, torch.float64,
+                                               weights=R.model_weights(0.0 if tc else 1.0), frozen_blocks=(0,),
+                                               forced_masks=masks)
+    bar_stats, bar_loss = (5e-5, 1e-4) if tc else (1e-5, 1e-5)          # tf32 measured 7.0e-6 / 2.4e-6 (B200)
     after = model.get_weights_dict()
     for k in w:
         if "Head_0/BatchNorm/moving" in k:
             assert (after[k] == w[k]).all(), f"{k}: a frozen head's moving statistics were updated"
         if "Head_1/BatchNorm/moving" in k:
-            assert nerr(after[k], stats[k]) < 1e-5, k
-    assert nerr(model.metric_tensors["loss"].cpu().numpy(), out["loss"].detach().numpy()) < 1e-5
+            print(f"  {k}: {nerr(after[k], stats[k]):.2e}")
+            assert nerr(after[k], stats[k]) < bar_stats, k
+    e_loss = nerr(model.metric_tensors["loss"].cpu().numpy(), out["loss"].detach().numpy())
+    print(f"  loss vector {e_loss:.2e}")
+    assert e_loss < bar_loss
     g = model.get_grads_dict()
+    frozen = [k for k in g if k.split("/")[0].endswith("_0")]
+    assert frozen
+    for k in frozen:
+        assert (after[k] == w[k]).all(), f"{k}: a frozen variable was updated"
+        if tc:      # the fused path computes no parameter gradient for a frozen block or head (gw / d_pos NULL)
+            assert not np.any(g[k]), f"{k}: a frozen variable received a gradient"
+    gmax = max(float(np.abs(v).max()) for v in grads.values())
+    worst = (0.0, None)
     for k, ref in grads.items():
         if ("_1/" in k or k.startswith("DecoderPrep")) and "KeyProjection/bias" not in k:      # (key bias: mathematically zero)
-            assert nerr(g[k], ref, 1e-6 * max(float(np.abs(v).max()) for v in grads.values())) < 5e-4, k
+            if tc:      # the tf32 gradient bar of test_model_train_step_tf32: relative L2 per tensor
+                e = float(np.linalg.norm(g[k] - ref) / max(np.linalg.norm(ref), 1e-30))
+            else:
+                e = nerr(g[k], ref, 1e-6 * gmax)
+            worst = max(worst, (e, k))
+    print(f"  worst block-1 / query gradient: {worst[1]} {worst[0]:.2e}")
+    assert worst[0] < (5e-2 if tc else 5e-4), worst[1]
 
 
 def test_bucketed_optimizer_equals_whole_buffer_update(tc_mode):

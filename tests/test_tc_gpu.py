@@ -9,6 +9,13 @@ from test_dense_gpu import _model_and_data, nerr
 pytestmark = pytest.mark.gpu
 
 
+def tf32(x):
+    """Round to nearest tf32 like the producers do (bdetr_round_tf32)."""
+    u = np.asarray(x).astype(np.float32).view(np.uint32).astype(np.uint64)
+    u = ((u + 0x1000) & 0xFFFFE000).astype(np.uint32)
+    return u.view(np.float32)
+
+
 @pytest.fixture()
 def tc_mode():
     from boosted_detr_b200 import _lib
@@ -31,6 +38,7 @@ def test_umma_gemm_variants(tc_mode):
         (1000, 192, 96, 0, 0, 1, 0, 0),       # odd sizes: N tail, K = 3 k-blocks
         (300, 64, 40, 0, 1, 0, 0, 0),         # K tail handled by TMA zero fill
         (128, 128, 32, 1, 1, 0, 0, 0),        # A MN-major, B K-major
+        (256, 296, 6400, 1, 0, 0, 0, 0),      # config-3 attribute head h^T d_logits: both MN-major, ragged N, split-K overwrite
     ]
     for (M, N, K, ta, tb, bias, act, beta) in cases:
         A = rng.standard_normal((K, M) if ta else (M, K)).astype(np.float32)
@@ -180,11 +188,6 @@ def test_attention_core_multistream(tc_mode, B, Lq, Lk, qscale):
     H, d = 8, 32
     D = H * d
     rng = np.random.default_rng(Lq + Lk)
-
-    def tf32(x):                                      # round to nearest tf32 like the producers do
-        u = x.astype(np.float32).view(np.uint32).astype(np.uint64)
-        u = ((u + 0x1000) & 0xFFFFE000).astype(np.uint32)
-        return u.view(np.float32)
 
     q, k, v = (tf32(rng.standard_normal((B, L, D))) for L in (Lq, Lk, Lk))
     q = tf32(q * qscale)
