@@ -45,6 +45,7 @@ typedef enum {
                            * fp16 kernel does not serve, and every backward, run exactly as in BDETR_MODE_TF32 (the Python
                            * layers hand ws16 over for inference forwards only). */
 
+/* 101: attention at head dim 64 (D/H = 64) besides 32 */
 int bdetr_version(void);
 const char *bdetr_last_error(void);
 /* Process-wide compute mode used by the dense entry points. */
@@ -188,8 +189,8 @@ typedef struct {
 
 /* AttentionBlock.call (transformers.py:139-151) with MultiheadAttention.call (:68-102) inside:
  *   out = LayerNorm_eps( query + Dropout( MHA(query,key,value) ) )
- * query [B,Lq,D] (also the residual), key/value [B,Lk,D]; H heads of width D/H; the attention
- * output is re-read as [B,Lq,D] WITHOUT permuting back (reference line :100).
+ * query [B,Lq,D] (also the residual), key/value [B,Lk,D]; H heads of width D/H, which must be 32 or 64 (other widths
+ * return BDETR_E_UNSUPPORTED); the attention output is re-read as [B,Lq,D] WITHOUT permuting back (reference line :100).
  * dropout_rate 0 disables dropout (inference); the keep mask is hash(idx ^ key) >= rate * 2^32 with
  * key = dropout_key when dropout_seed_dev is NULL, else key = lowbias32(*dropout_seed_dev ^ dropout_key): the
  * per-step seed is then read from DEVICE memory by the kernels, so a captured CUDA graph draws a fresh mask on every
@@ -201,7 +202,7 @@ int bdetr_attention_block_fwd(int B, int Lq, int Lk, int D, int H,
                               const bdetr_attn_saved *saved, void *stream);
 
 /* The attention core alone (transformers.py:77-97): qp [B,Lq,H*d], kp/vp [B,Lk,H*d] are the projected tensors
- * (head = d-column slice), o [B,H,Lq,d], lse [B,H,Lq] (log2 units).  Scores are never written to HBM.
+ * (head = d-column slice), o [B,H,Lq,d], lse [B,H,Lq] (log2 units); d = 32 or 64.  Scores are never written to HBM.
  * Tensor-core mode runs the tcgen05/TMEM flash kernel; fp32 mode the SIMT kernel. */
 int bdetr_attention_core_fwd(int B, int H, int Lq, int Lk, int d, const float *qp, const float *kp, const float *vp,
                              float *o, float *lse, void *stream);
@@ -418,7 +419,9 @@ int bdetr_heads_bwd(int M, int D, int Dh, int C, int A, const float *x, const bd
 int bdetr_debug_set_timeline(long long *device_buf8);
 /* Debug / test aid: which tcgen05 attention-forward kernel the tensor-core mode uses.  0 = automatic (multi-stream
  * kernel for long sequences, one tile per CTA otherwise), 1 = always one tile per CTA, 2 = always multi-stream;
- * 20 + n = multi-stream with n of every 8 exponential groups evaluated on the FMA pipe. */
+ * 20 + n = multi-stream with n of every 8 exponential groups evaluated on the FMA pipe.  The multi-stream kernel serves
+ * head dim 32 only: at head dim 64 the automatic choice is the one-tile kernel, and forcing 2 or 20 + n makes the
+ * attention forward return BDETR_E_UNSUPPORTED without launching anything. */
 int bdetr_debug_force_attention_kernel(int which);
 
 /* Generic row-major GEMM used by the entry points above, exported for tests and benchmarks:
