@@ -153,7 +153,7 @@ extern "C" __attribute__((visibility("default"))) int bdetr_get_concurrency(void
 extern "C" __attribute__((visibility("default"))) int bdetr_set_deferred_join(int on) { bdetr::g_defer.store(on ? 1 : 0); return BDETR_OK; }
 extern "C" __attribute__((visibility("default"))) int bdetr_join(void *stream) { return bdetr::join_pending(reinterpret_cast<cudaStream_t>(stream), reinterpret_cast<cudaStream_t>(stream)); }
 extern "C" __attribute__((visibility("default"))) int bdetr_join_into(void *stream, void *waiter) { return bdetr::join_pending(reinterpret_cast<cudaStream_t>(stream), reinterpret_cast<cudaStream_t>(waiter)); }
-extern "C" __attribute__((visibility("default"))) int bdetr_version(void) { return 101; }
+extern "C" __attribute__((visibility("default"))) int bdetr_version(void) { return 102; }
 extern "C" __attribute__((visibility("default"))) const char *bdetr_last_error(void) { return bdetr::g_err; }
 extern "C" __attribute__((visibility("default"))) int bdetr_set_mode(int mode)
 {

@@ -94,6 +94,10 @@ struct HeadsOutArgs {
     const float *cum_in[3]; float *cum_out[3]; float *act[3];
 };
 constexpr int HO_ROWS = 32, HO_RPW = 4, HO_WBUF = 44 * 1024, HO_THREADS = 256;   // rows per CTA, rows per warp, bytes per W2 chunk buffer
+// Heads wider than HO_SLAB outputs: column slabs of HO_SLAB, W2 rows staged at stride HO_SLDW (the slab plus the
+// 16-byte alignment slack on both sides), HO_SCK rows per chunk (one bulk copy per lane of warp 0)
+constexpr int HO_SLAB = 320, HO_SLDW = HO_SLAB + 8, HO_SCK = 32, HO_MAXN = 2048;
+static_assert(HO_SCK * HO_SLDW * 4 <= HO_WBUF, "slab chunk must fit one W2 buffer");
 
 __device__ __forceinline__ float sigmoidf_h(float x) { return 1.0f / (1.0f + expf(-x)); }
 
@@ -104,10 +108,30 @@ __device__ __forceinline__ void bulk_load_1d(void *dst, const void *src, uint32_
                  ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
-// rows of this warp (HO_RPW + the shift row) x NJ output columns per lane, W2 streamed in row chunks of CK hidden units
-template <int NJ>
+// Slab path: W2 rows c1 .. c1 + ck - 1 (ck <= 32), columns [n0, n0 + w), into dst at row stride HO_SLDW.  A slab row is
+// not 16-byte aligned in general (row stride N), so lane i copies the aligned span that covers row c1 + i; the slab
+// starts (c N + n0) & 3 floats into it.  The span never passes the end of W2: Dh N is a multiple of 4.
+__device__ __forceinline__ void heads_slab_chunk(const float *w2, int N, int n0, int w, int c1, int ck, float *dst, uint64_t *bar)
+{
+    const int lane = threadIdx.x & 31;
+    size_t s0 = 0;
+    uint32_t bytes = 0;
+    if (lane < ck) {
+        const size_t st = (size_t)(c1 + lane) * N + n0;
+        s0 = st & ~size_t(3);
+        bytes = (uint32_t)((((st + w + 3) & ~size_t(3)) - s0) * 4);
+    }
+    const uint32_t total = __reduce_add_sync(0xffffffffu, bytes);
+    if (lane == 0) mbar_expect_tx(bar, total);
+    __syncwarp();
+    if (lane < ck) bulk_load_1d(dst + lane * HO_SLDW, w2 + s0, bytes, bar);
+}
+
+// rows of this warp (HO_RPW + the shift row) x NJ output columns per lane, W2 streamed in row chunks of CK hidden units.
+// SLAB: columns [n0, n0 + w) of a wider head (CK = HO_SCK); the raw logits go to act, the row activation runs after.
+template <int NJ, bool SLAB = false>
 __device__ __forceinline__ void heads_out_rows(const HeadsOutArgs &a, int k, int N, int M, int Dh, int m0, const float *sH, float *sWbuf,
-                                               uint64_t *bars, int CK)
+                                               uint64_t *bars, int CK, int n0 = 0, int w = 0)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const float *w2 = a.w2[k];
@@ -118,14 +142,24 @@ __device__ __forceinline__ void heads_out_rows(const HeadsOutArgs &a, int k, int
         for (int j = 0; j < NJ; ++j) acc[r][j] = 0.0f;
     const float *hr = sH + (warp * HO_RPW) * Dh, *hs = sH + HO_ROWS * Dh;
     const int nchunks = (Dh + CK - 1) / CK;
-    if (threadIdx.x == 0) {
+    const int ldw = SLAB ? HO_SLDW : N;
+    int off[4] = {0, 0, 0, 0};                                // SLAB: where the slab starts in a staged row (chunks start at multiples of 4 rows)
+    if (SLAB) {
+#pragma unroll
+        for (int cc = 0; cc < 4; ++cc) off[cc] = (cc * N + n0) & 3;
+        if (warp == 0) heads_slab_chunk(w2, N, n0, w, 0, min(CK, Dh), sWbuf, &bars[0]);
+    } else if (threadIdx.x == 0) {
         const int ck = min(CK, Dh);
         mbar_expect_tx(&bars[0], (uint32_t)(ck * N * 4));
         bulk_load_1d(sWbuf, w2, (uint32_t)(ck * N * 4), &bars[0]);
     }
     for (int ch = 0; ch < nchunks; ++ch) {
         const int c0 = ch * CK, ck = min(CK, Dh - c0);
-        if (threadIdx.x == 0 && ch + 1 < nchunks) {          // next chunk into the other buffer (its readers passed the barrier below)
+        if (SLAB) {
+            if (warp == 0 && ch + 1 < nchunks)
+                heads_slab_chunk(w2, N, n0, w, c0 + CK, min(CK, Dh - c0 - CK),
+                                 reinterpret_cast<float *>(reinterpret_cast<uint8_t *>(sWbuf) + ((ch + 1) & 1) * HO_WBUF), &bars[(ch + 1) & 1]);
+        } else if (threadIdx.x == 0 && ch + 1 < nchunks) {   // next chunk into the other buffer (its readers passed the barrier below)
             const int c1 = c0 + CK, ck1 = min(CK, Dh - c1);
             mbar_expect_tx(&bars[(ch + 1) & 1], (uint32_t)(ck1 * N * 4));
             bulk_load_1d(reinterpret_cast<uint8_t *>(sWbuf) + ((ch + 1) & 1) * HO_WBUF, w2 + (size_t)c1 * N, (uint32_t)(ck1 * N * 4), &bars[(ch + 1) & 1]);
@@ -139,7 +173,7 @@ __device__ __forceinline__ void heads_out_rows(const HeadsOutArgs &a, int k, int
             hv[HO_RPW] = *reinterpret_cast<const float4 *>(hs + c0 + c);
 #pragma unroll
             for (int cc = 0; cc < 4; ++cc) {
-                const float *wrow = sW + (c + cc) * N + lane;
+                const float *wrow = sW + (c + cc) * ldw + off[cc] + lane;
                 float w[NJ];
 #pragma unroll
                 for (int j = 0; j < NJ; ++j) w[j] = wrow[32 * j];           // (columns >= N read the next row / slack: discarded below)
@@ -155,6 +189,19 @@ __device__ __forceinline__ void heads_out_rows(const HeadsOutArgs &a, int k, int
     }
     // logits = acc[row] + (shift W2 + b2); activation; running sum
     float bb[NJ];
+    if (SLAB) {
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) bb[j] = (lane + 32 * j < w) ? a.b2[k][n0 + lane + 32 * j] + acc[HO_RPW][j] : 0.0f;
+#pragma unroll
+        for (int r = 0; r < HO_RPW; ++r) {
+            const int m = m0 + warp * HO_RPW + r;
+            if (m >= M) continue;
+#pragma unroll
+            for (int j = 0; j < NJ; ++j)
+                if (lane + 32 * j < w) a.act[k][(size_t)m * N + n0 + lane + 32 * j] = acc[r][j] + bb[j];
+        }
+        return;
+    }
 #pragma unroll
     for (int j = 0; j < NJ; ++j) bb[j] = (lane + 32 * j < N) ? a.b2[k][lane + 32 * j] + acc[HO_RPW][j] : 0.0f;
 #pragma unroll
@@ -195,12 +242,17 @@ __device__ __forceinline__ void heads_out_rows(const HeadsOutArgs &a, int k, int
 // columns lane, lane + 32, ...  BatchNorm is applied while the rows are staged (sH = h * scale; one extra row holds
 // `shift`, whose product with W2 is the folded bias), so hn is never materialised.  W2 [Dh, N] arrives in row chunks by TMA
 // bulk copies (double-buffered).  dynamic smem: bars | sH [33][Dh] | sW 2 x 44 KB (+ slack)
+// SLABS (some head has more than HO_SLAB outputs): grid.z = column slabs.  A head that wide gets its raw logits, slab by
+// slab, from every z; a narrower head runs the whole-row path above in z = 0 only.
+template <bool SLABS>
 __global__ void __launch_bounds__(HO_THREADS)
 heads_out_kernel(HeadsOutArgs a)
 {
     extern __shared__ __align__(128) uint8_t smem_b[];
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem_b);
     const int k = blockIdx.y, Dh = a.d.Dh, N = a.d.n[k], M = a.d.M;
+    const int n0 = SLABS ? blockIdx.z * HO_SLAB : 0;
+    if (SLABS && (N > HO_SLAB ? n0 >= N : blockIdx.z != 0)) return;
     float *sH = reinterpret_cast<float *>(smem_b + 128);
     float *sW = sH + (HO_ROWS + 1) * Dh;
     if (threadIdx.x == 0) {
@@ -223,6 +275,10 @@ heads_out_kernel(HeadsOutArgs a)
         *reinterpret_cast<float4 *>(sH + r * Dh + 4 * c4) = v;
     }
     __syncthreads();
+    if (SLABS && N > HO_SLAB) {
+        heads_out_rows<10, true>(a, k, N, M, Dh, m0, sH, sW, bars, HO_SCK, n0, min(HO_SLAB, N - n0));
+        return;
+    }
     // rows of W2 per chunk: a multiple of 4 (16-byte sized / aligned copies) that fits one 48 KB buffer
     const int CK = max(4, min(Dh, (HO_WBUF / (N * 4)) & ~3));
     if (N <= 32) heads_out_rows<1>(a, k, N, M, Dh, m0, sH, sW, bars, CK);
@@ -404,7 +460,7 @@ API int bdetr_heads_fwd(int M, int D, int Dh, int C, int A, const float *x, cons
 {
     HeadsDims d;
     BDETR_REQUIRE(heads_dims(d, M, Dh, C, A) && D > 0 && D % 4 == 0, BDETR_E_BAD_SHAPE, "bad shape (hidden width <= 256)");
-    BDETR_REQUIRE(C <= 320 && A <= 320, BDETR_E_UNSUPPORTED, "fused heads: at most 320 outputs per head");
+    BDETR_REQUIRE(C <= HO_MAXN && A <= HO_MAXN, BDETR_E_UNSUPPORTED, "fused heads: at most 2048 outputs per head");
     BDETR_REQUIRE(x && heads && bn_training && cum_out && sv && sv->h && sv->bn_mean && sv->bn_rstd && sv->bn_part && sv->w2f && sv->b2f, BDETR_E_NULL, "null pointer");
     ModeScope tc(BDETR_MODE_TF32);
     cudaStream_t s = as_stream(stream);
@@ -437,13 +493,24 @@ API int bdetr_heads_fwd(int M, int D, int Dh, int C, int A, const float *x, cons
         o.cum_in[k] = cum_in ? cum_in[k] : nullptr; o.cum_out[k] = cum_out[k]; o.act[k] = sv->act[k];
     }
     const size_t smem = 128 + (size_t)(HO_ROWS + 1) * Dh * sizeof(float) + 2 * HO_WBUF + 2048;
-    static size_t optin = 0;
-    if (smem > optin) {
-        BDETR_CUDA(cudaFuncSetAttribute(heads_out_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        optin = smem;
+    const int slabs = ceil_div(max(C, A), HO_SLAB);
+    auto kern = slabs > 1 ? heads_out_kernel<true> : heads_out_kernel<false>;
+    static size_t optin[2] = {0, 0};
+    if (smem > optin[slabs > 1]) {
+        BDETR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        optin[slabs > 1] = smem;
     }
-    launch_k(heads_out_kernel, dim3(ceil_div(M, HO_ROWS), 3), HO_THREADS, smem, s, o);
+    launch_k(kern, dim3(ceil_div(M, HO_ROWS), 3, slabs), HO_THREADS, smem, s, o);
     BDETR_CHECK_LAUNCH("heads_out_kernel");
+    // heads wider than a slab: activation over the whole row and the running sum, in the per-row order of the layer path
+    for (int k = 0; k < 2; ++k) {
+        const int n = d.n[k];
+        if (n <= HO_SLAB) continue;
+        const bool have_in = cum_in && cum_in[k];
+        if (have_in && cum_in[k] != cum_out[k])
+            BDETR_CUDA(cudaMemcpyAsync(cum_out[k], cum_in[k], sizeof(float) * M * n, cudaMemcpyDeviceToDevice, s));
+        TRY(launch_head_act_fwd(M, n, k, mult, sv->act[k], cum_out[k], have_in ? 0 : 1, s));
+    }
     return BDETR_OK;
 }
 
@@ -466,12 +533,16 @@ API int bdetr_heads_bwd(int M, int D, int Dh, int C, int A, const float *x, cons
     const int nmax = max(max(C, A), 4);
     launch_k(heads_act_bwd_kernel, dim3(ceil_div(M, 32), 3), 256, sizeof(float) * nmax, s, ab);
     BDETR_CHECK_LAUNCH("heads_act_bwd_kernel");
-    // G[k] = h[k]^T d_logits[k]  ([Dh, n_k], contraction over the M rows)
+    // G[k] = h[k]^T d_logits[k]  ([Dh, n_k], contraction over the M rows).  A head wider than a slab takes the fp32
+    // GEMM: with tf32 operands the second-layer weight and BatchNorm gamma gradients of a 2048-output head were off by
+    // 1e-3 of their largest value (1e-6 in fp32).
     {
         Branches br(s);
-        for (int k = 0; k < 3; ++k)
+        for (int k = 0; k < 3; ++k) {
+            ModeScope gm(d.n[k] > HO_SLAB ? BDETR_MODE_FP32 : BDETR_MODE_TF32);
             TRY(launch_gemm(Dh, d.n[k], M, sv->h + k * hs, Dh, true, sc->d_logits + (size_t)M * d.off[k], d.n[k], false, nullptr, 0, nullptr,
                             0, 0, sc->hTd + (size_t)Dh * d.off[k], d.n[k], k == 0 ? s : br.fork(k - 1)));
+        }
         TRY(br.join());
     }
     HeadsBnBwdArgs bb;

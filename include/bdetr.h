@@ -99,7 +99,18 @@ int bdetr_cost_matrix_fwd(int B, int T, int Q, int C, int A,
  *                               bdetr_cost_targets_bytes(B,T,C,A) bytes, 16-byte aligned;
  *   bdetr_cost_matrix_prepared  builds cost[B,T,Q] from it; bit-identical to bdetr_cost_matrix_fwd.
  * bdetr_cost_matrix_fwd itself is these two calls on a library-owned grow-only scratch buffer (allocated on first use,
- * outside graph capture; one buffer per device, so not for concurrent use from several streams). */
+ * outside graph capture; one buffer per device, so not for concurrent use from several streams).
+ * Limits (BDETR_E_UNSUPPORTED, before anything is launched):
+ *   prepare   C <= 2048, A <= 1024, T*C and T*A < 2^22.  The target blocks are staged in shared memory when
+ *             T*(C+A) floats plus the digest fit 227 KB and C <= 1024; otherwise they are read from global memory.
+ *   cost      C <= 2048.  With Cs = C|1 and As = A|1, the cost tile takes
+ *                 16 + 256*C (16-byte aligned) + digest + 256*Cs + attr + 256  bytes,
+ *             digest = bdetr_cost_targets_bytes(1,T,C,A), attr = 0 when w_attr == 0, else 256*17 for A <= 4 and
+ *             256*As above.  When that exceeds 227 KB the 256*C tile is dropped and 256*Cs becomes
+ *             256*(min(C,T)|1) (the probabilities of the classes that occur are read from global memory); the call
+ *             is refused if that still exceeds 227 KB, which only a large A can cause (A above about 620 at T = 100 and
+ *             C = 2048, about 840 at T = 20 and C = 1205).
+ *   Both paths give the same bits. */
 size_t bdetr_cost_targets_bytes(int B, int T, int C, int A);
 int bdetr_cost_targets_prepare(int B, int T, int C, int A,
                                const float *cat_true, const float *attr_true, const float *box_true,
@@ -388,7 +399,9 @@ int bdetr_decoder_self_bwd(int B, int Q, int D, int H, const float *q0, const fl
  * heads[0..2] = category (softmax, Nout = C), attribute (sigmoid, A), box (3*sigmoid(x/100)-1, 4).
  *   saved: h [3,M,Dh] post-ReLU hidden activations, bn_mean / bn_rstd [3,Dh], w2f / b2f [3,Dh] the affine map
  *   hn = h * w2f + b2f the output kernel folds into the second Dense, bn_part scratch, act[k] [M,Nout_k] post-activation
- *   outputs.  C, A <= 320.
+ *   outputs.  C, A <= 2048 (BDETR_E_UNSUPPORTED above, before anything is launched).  A head of more than 320
+ *   outputs computes its logits in column slabs of 320 and then runs the row activation and the running sum as a
+ *   second kernel; narrower heads run the one-kernel path.
  * bn_training[k] = 0: head k normalises with its moving statistics (inference, or a frozen head). */
 typedef struct {
     float *h, *bn_mean, *bn_rstd, *w2f, *b2f;
