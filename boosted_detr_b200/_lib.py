@@ -4,7 +4,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import POINTER, Structure, c_float, c_int, c_int32, c_longlong, c_size_t, c_uint32, c_void_p, c_char_p
+from ctypes import POINTER, Structure, c_float, c_int, c_int32, c_longlong, c_size_t, c_uint32, c_ulonglong, c_void_p, c_char_p
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libbdetr.so")
@@ -106,6 +106,12 @@ PROTOTYPES = {
     "bdetr_backbone_neck_fwd": (c_int, [I, I, I, P, POINTER(NeckParams), F, F, I, P, POINTER(NeckSaved), I, P]),
     "bdetr_backbone_neck_bwd": (c_int, [I, I, I, P, POINTER(NeckParams), I, POINTER(NeckSaved), P, POINTER(NeckParams), P, P, P]),
     "bdetr_inverse_tokenize": (c_int, [I, I, I, I, P, P, P, P, P, P, F, P]),
+    "bdetr_exit_graph_create": (c_int, [I, POINTER(c_void_p), POINTER(c_ulonglong)]),
+    "bdetr_exit_graph_build": (c_int, [P, POINTER(c_void_p), I]),
+    "bdetr_exit_graph_launch": (c_int, [P, P]),
+    "bdetr_exit_graph_destroy": (c_int, [P]),
+    "bdetr_early_exit_decide": (c_int, [I, I, I, P, P, P, P, c_ulonglong, P, P, P]),
+    "bdetr_select_exit_predictions": (c_int, [I, I, I, I, I, POINTER(c_void_p), P, P, P, P, P]),
     "bdetr_comm_unique_id": (c_int, [P]),
     "bdetr_comm_init": (c_int, [POINTER(c_void_p), I, I, P]),
     "bdetr_comm_destroy": (c_int, [P]),

@@ -85,6 +85,7 @@ class BoostedDETR:
         self.early_exit_threshold = None
         self.early_exit_min_blocks = 1
         self.last_exit_block = None
+        self._exit_capture = None         # set by graph.GraphedInference while it captures the forward in segments
         self.step_count = 0
         self.num_replicas = 1
         self.grad_allreduce = None        # set by parallel.DataParallel (joins / performs the gradient all-reduce)
@@ -388,6 +389,15 @@ class BoostedDETR:
         self.last_image_confidence = self._exit_host.clone()
         return bool((self._exit_host >= self.early_exit_threshold).all())
 
+    def _exit_boundary(self, i, cums, streams):
+        """True when the inference forward stops after boosted block i (`_early_exit`).  While graph.GraphedInference
+        captures the forward in segments, the decision is a captured kernel instead and every block is issued: it ends
+        the current segment there, after joining `streams` (every stream the forward has forked), and begins the next."""
+        if self._exit_capture is None:
+            return self._early_exit(i, cums)
+        self._exit_capture.boundary(i, cums, streams)
+        return False
+
     # -- fused tensor-core path -------------------------------------------------------------------
     def _use_fused(self, feats):
         """Tensor-core mode, model width 256, every layer already built (the very first call builds the layers lazily
@@ -474,7 +484,8 @@ class BoostedDETR:
             keys = self._keys(i) if use_dropout else None
             enc, dec_l = self.EncoderTransformerBlocks[i], self.DecoderBlocks[i]
             dkeys = keys["dec"] if keys else (0, 0, 0)
-            main.wait_event(pre_ev[i])
+            if pre_ev[i] is not None:
+                main.wait_event(pre_ev[i])
             (x, pos), c_enc = enc.forward([x], training, keys["enc"] if keys else None, seed_dev, tabs=tabs[i][:2])
             self._mark(f"fwd enc{i} done (main)")
             bs = bstreams[i]
@@ -497,8 +508,13 @@ class BoostedDETR:
                     loss_ctxs.append(self.loss_fn.forward(y_true, cums, prepared))
                     self._mark(f"fwd loss{i} done (side)")
                 self.last_exit_block = i
-                if not training and self._early_exit(i, cums):
-                    break
+                if not training:
+                    if self._exit_boundary(i, cums, [main, pre_s, *bstreams]):
+                        break
+                    if self._exit_capture is not None:
+                        # a new graph segment has begun behind a join of every stream: events recorded in the previous
+                        # segments cannot be waited on, and the join already orders everything after them
+                        heads_ev, pre_ev = None, [None] * N
         for bs in bstreams:
             main.wait_stream(bs)
         main.wait_stream(pre_s)
@@ -755,7 +771,7 @@ class BoostedDETR:
                 cums = new_cums
                 blocks.append({"enc": c_enc, "prep": c_prep, "dec": c_dec, "heads": c_heads})
                 self.last_exit_block = i
-                if not training and self._early_exit(i, cums):
+                if not training and self._exit_boundary(i, cums, [main, *aux]):
                     break
                 if training:
                     ls = loss_streams[i]

@@ -1,11 +1,16 @@
 """CUDA-graph replay of the training step: the whole fwd + matcher + bwd chain is ~600 small kernels, so at
-BASELINE config 2 the step is launch-bound; one graph launch replaces the Python/ctypes launch sequence."""
+BASELINE config 2 the step is launch-bound; one graph launch replaces the Python/ctypes launch sequence.
+GraphedInference does the same for BoostedDETR.call(training=False), with the early exit decided on the device."""
 from __future__ import annotations
+
+import ctypes
+import time
 
 import numpy as np
 import torch
 
-from .device import ptr
+from . import _lib
+from .device import empty, ptr, require_cuda, stream_ptr
 from .losses_and_metrics import raise_for_status
 
 
@@ -158,3 +163,255 @@ class GraphedTrainStep:
         if not return_host:
             return self.metrics
         return self.model.host_logs()
+
+
+def _is_capturing(stream):
+    with torch.cuda.stream(stream):
+        return torch.cuda.is_current_stream_capturing()
+
+
+class GraphedInference:
+    """Captures BoostedDETR.call(training=False) for one input shape and compute mode.  `__call__(inputs)` copies
+    `features` (or `backbone_features` for a model with a backbone neck) into a static input buffer, replays and returns
+    the three running predictions [cat, attr, box].  Those tensors are static buffers: the next call overwrites them
+    (clone them to keep a result).  Inputs may be CUDA tensors, pinned host tensors or numpy arrays (through the model's
+    pinned staging), as in GraphedTrainStep.load.
+
+    The capture shape is fixed by `model.early_exit_threshold` at construction:
+      None      one graph around the forward, with its multi-stream schedule across blocks as is;
+      a number  the forward captured in segments (S0 = prologue + block 0, Sk = block k + the device-side exit decision
+                after it, E = the output select), stitched by the library into
+                    S0 -> IF(h0){S1} -> IF(h1){S2} -> ... -> E
+                so the blocks after the exit block do not run (include/bdetr.h "Graph-captured inference").  The threshold
+                and `early_exit_min_blocks` live in device words: a change takes effect at the next call, without a new
+                capture.  Switching between None and a number needs a new GraphedInference.
+    `last_exit_block` and `last_image_confidence` are read from the device on first access after a call and equal what
+    the eager call leaves on the model (`last_image_confidence` is None when no block boundary was checked)."""
+
+    def __init__(self, model, example_inputs, warmup=2):
+        self.model = model
+        if model._flat is None:
+            model.build()
+        lib = _lib.load()
+        self.mode = lib.bdetr_get_mode()
+        self.key = "backbone_features" if model.BackboneNeck is not None and "backbone_features" in example_inputs else "features"
+        self.shape = tuple(example_inputs[self.key].shape)
+        self.static_in = torch.empty(self.shape, dtype=torch.float32, device=require_cuda())
+        self.segmented = model.early_exit_threshold is not None
+        N, B, Q = model.num_decoder_blocks, self.shape[0], model.num_object_preds
+        self.load(example_inputs)
+        self._exit_graph = None
+        if self.segmented:
+            # device words the decide kernels read: threshold (float32), min_blocks, threshold set; the exit block; the
+            # image confidences of every boundary
+            self._thr_dev = torch.zeros(1, dtype=torch.float32, device=require_cuda())
+            self._int_dev = torch.zeros(2, dtype=torch.int32, device=require_cuda())
+            self._exit_dev = torch.full((1,), N - 1, dtype=torch.int32, device=require_cuda())
+            self._conf_dev = torch.zeros(max(N - 1, 1), B, dtype=torch.float32, device=require_cuda())
+            self._conf_q, self._iconf = empty(B, Q), empty(B)
+            self._words = None
+            self.out = [empty(B, Q, n) for n in (model.num_categories, model.num_attributes, 4)]
+        saved_thr, saved_trace = model.early_exit_threshold, getattr(model, "_trace", None)
+        model._trace = None                        # no timing-event nodes: a conditional body may not hold event nodes
+        try:
+            model.early_exit_threshold = None      # warm-up: every block, no host-side exit
+            side = torch.cuda.Stream()
+            side.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(side):
+                for _ in range(warmup):
+                    cums = self._forward()[0]
+                if self.segmented:                 # load the decide / select kernels outside the capture
+                    self._cums = [cums] * N
+                    if N > 1:
+                        self._decide(0, cums, 0)
+                    self._select()
+            torch.cuda.current_stream().wait_stream(side)
+            torch.cuda.synchronize()
+            model.early_exit_threshold = saved_thr
+            t0 = time.perf_counter()
+            if self.segmented:
+                self._capture_segments()
+            else:
+                self.graph = torch.cuda.CUDAGraph(keep_graph=True)
+                with torch.cuda.graph(self.graph):
+                    self.out, self._keep = self._forward()
+            t1 = time.perf_counter()
+            if self.segmented:
+                segs = (ctypes.c_void_p * len(self._segs))(*[g.raw_cuda_graph() for g in self._segs])
+                _lib.check(lib.bdetr_exit_graph_build(self._exit_graph, segs, len(self._segs)))
+            else:
+                self.graph.instantiate()
+            torch.cuda.synchronize()
+            self.capture_seconds, self.instantiate_seconds = t1 - t0, time.perf_counter() - t1
+        finally:
+            model.early_exit_threshold, model._trace = saved_thr, saved_trace
+            model._exit_capture = None
+        self._host = None
+        self._read = None
+
+    def _forward(self):
+        feats, _ = self.model._prepare({self.key: self.static_in}, False)
+        cums, ctx = self.model.forward(feats, None, False)
+        return cums, (feats, ctx)
+
+    # -- segmented capture ------------------------------------------------------------------------------------------
+    def _capture_segments(self):
+        m = self.model
+        lib = _lib.load()
+        N = m.num_decoder_blocks
+        handles = (ctypes.c_ulonglong * max(N - 1, 1))()
+        g = ctypes.c_void_p()
+        _lib.check(lib.bdetr_exit_graph_create(N - 1, ctypes.byref(g), handles))
+        self._exit_graph, self._handles = g, list(handles)[:N - 1]
+        self._pool = torch.cuda.graph_pool_handle()
+        self._origin = torch.cuda.Stream()
+        self._origin.wait_stream(torch.cuda.current_stream())
+        self._segs, self._cums = [], []
+        with torch.cuda.stream(self._origin):
+            self._begin_segment()
+            m._exit_capture = self
+            try:
+                cums, self._keep = self._forward()
+            finally:
+                m._exit_capture = None
+            assert len(self._cums) == N and self._cums[-1] is cums
+            self._segs[-1].capture_end()
+            self._begin_segment()
+            self._select()
+            self._segs[-1].capture_end()
+
+    def _begin_segment(self):
+        g = torch.cuda.CUDAGraph(keep_graph=True)
+        g.capture_begin(pool=self._pool)
+        self._segs.append(g)
+
+    def _decide(self, i, cums, handle):
+        """Image confidences of boundary i, exactly as BoostedDETR._early_exit computes them, and the decision kernel."""
+        N = self.model.num_decoder_blocks
+        B, Q, C = cums[0].shape
+        _lib.call("bdetr_inverse_tokenize", B, Q, C, cums[1].shape[-1], ptr(cums[0]), None, None, None, ptr(self._conf_q),
+                  ptr(self._iconf), 1.0 / (i + 2), stream_ptr())
+        _lib.call("bdetr_early_exit_decide", B, i, N, ptr(self._iconf), ptr(self._thr_dev), ptr(self._int_dev[0:1]),
+                  ptr(self._int_dev[1:2]), handle, ptr(self._exit_dev), ptr(self._conf_dev[i]), stream_ptr())
+
+    def _select(self):
+        m = self.model
+        B, Q = self.out[0].shape[:2]
+        srcs = (ctypes.c_void_p * (3 * len(self._cums)))(*[c.data_ptr() for cums in self._cums for c in cums])
+        _lib.call("bdetr_select_exit_predictions", len(self._cums), B, Q, m.num_categories, m.num_attributes, srcs,
+                  ptr(self._exit_dev), ptr(self.out[0]), ptr(self.out[1]), ptr(self.out[2]), stream_ptr())
+
+    def boundary(self, i, cums, streams):
+        """Called by the forward after boosted block i (BoostedDETR._exit_boundary) while the segments are captured:
+        queues the decision for block i + 1 on the stream that produced `cums`, joins every forked stream into the
+        capture's origin stream, ends segment i and begins segment i + 1 there, and forks the same streams again."""
+        self._cums.append(cums)
+        if i + 1 >= self.model.num_decoder_blocks:
+            return
+        self._decide(i, cums, self._handles[i])
+        origin, forked = self._origin, []
+        for s in [torch.cuda.current_stream(), *streams]:
+            if s != origin and s not in forked and _is_capturing(s):
+                origin.wait_stream(s)
+                forked.append(s)
+        with torch.cuda.stream(origin):
+            self._segs[-1].capture_end()
+            self._begin_segment()
+        for s in forked:
+            s.wait_stream(origin)
+
+    def _push_words(self):
+        """Queues the exit settings on the current stream when they changed (fills, no host buffer involved).  Eager
+        compares the float32 confidences with the threshold in float32: it is rounded to float32 once, here."""
+        m = self.model
+        words = (float(np.float32(m.early_exit_threshold)), int(m.early_exit_min_blocks))
+        if words != self._words:
+            self._thr_dev.fill_(words[0])
+            self._int_dev[0:1].fill_(words[1])
+            self._int_dev[1:2].fill_(1)
+            self._words = words
+
+    # -- calls ------------------------------------------------------------------------------------------------------
+    def _check(self, inputs):
+        m = self.model
+        if self.key not in inputs:
+            raise KeyError(f"GraphedInference was captured for inputs['{self.key}']")
+        shape = tuple(inputs[self.key].shape)
+        if shape != self.shape:
+            raise ValueError(f"GraphedInference was captured for {self.key} of shape {self.shape}, got {shape}: "
+                             "capture a new GraphedInference for this shape")
+        mode = _lib.load().bdetr_get_mode()
+        if mode != self.mode:
+            raise RuntimeError(f"GraphedInference was captured in compute mode {self.mode}, the library is in mode {mode}: "
+                               "capture a new GraphedInference in this mode")
+        if (m.early_exit_threshold is not None) != self.segmented:
+            raise RuntimeError("early_exit_threshold changed between None and a number since the capture: the early exit "
+                               "needs a differently shaped graph, capture a new GraphedInference")
+
+    def load(self, inputs):
+        """Host or device input -> the static input buffer, async on the current stream."""
+        x, dst = inputs[self.key], self.static_in
+        m = self.model
+        m.h2d_bytes = 0
+        if isinstance(x, torch.Tensor) and x.is_cuda:
+            if x.data_ptr() != dst.data_ptr():
+                dst.copy_(x.reshape(dst.shape), non_blocking=True)
+        elif isinstance(x, torch.Tensor) and x.is_pinned() and x.dtype == dst.dtype and x.is_contiguous():
+            dst.copy_(x.reshape(dst.shape), non_blocking=True)
+            m.h2d_bytes += x.numel() * x.element_size()
+        else:
+            m._h2d(self.key, x, "f32", dst=dst)
+
+    def replay(self):
+        if self.segmented:
+            self._push_words()
+            _lib.check(_lib.load().bdetr_exit_graph_launch(self._exit_graph, stream_ptr()))
+        else:
+            self.graph.replay()
+        self._read = None
+
+    def __call__(self, inputs, return_host=False):
+        self._check(inputs)
+        self.load(inputs)
+        self.replay()
+        if not return_host:
+            return self.out
+        if self._host is None:
+            self._host = [torch.empty(t.shape, dtype=t.dtype).pin_memory() for t in self.out]
+        for h, t in zip(self._host, self.out):
+            h.copy_(t, non_blocking=True)
+        torch.cuda.current_stream().synchronize()
+        return [h.numpy().copy() for h in self._host]
+
+    def _exit_state(self):
+        if self._read is None:
+            m = self.model
+            N = m.num_decoder_blocks
+            if not self.segmented:
+                self._read = (N - 1, None)
+            else:
+                e = int(self._exit_dev.item())
+                # the boundaries eager checks: min_blocks - 1 .. N - 2, up to the exit
+                last = e if e < N - 1 else N - 2
+                conf = self._conf_dev[last].cpu() if last >= max(self._words[1] - 1, 0) else None
+                self._read = (e, conf)
+        return self._read
+
+    @property
+    def last_exit_block(self):
+        return self._exit_state()[0]
+
+    @property
+    def last_image_confidence(self):
+        return self._exit_state()[1]
+
+    def close(self):
+        if self._exit_graph is not None:
+            _lib.check(_lib.load().bdetr_exit_graph_destroy(self._exit_graph))
+            self._exit_graph = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

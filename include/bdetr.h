@@ -45,7 +45,8 @@ typedef enum {
                            * fp16 kernel does not serve, and every backward, run exactly as in BDETR_MODE_TF32 (the Python
                            * layers hand ws16 over for inference forwards only). */
 
-/* 101: attention at head dim 64 (D/H = 64) besides 32 */
+/* 101: attention at head dim 64 (D/H = 64) besides 32
+ * 103: graph-captured inference with the early exit on the device (bdetr_exit_graph_*, bdetr_early_exit_decide) */
 int bdetr_version(void);
 const char *bdetr_last_error(void);
 /* Process-wide compute mode used by the dense entry points. */
@@ -502,6 +503,40 @@ int bdetr_backbone_neck_bwd(int M, int Cin, int N, const float *x_tc, const bdet
 int bdetr_inverse_tokenize(int B, int Q, int C, int A, const float *cat_pred, const float *attr_pred,
                            int32_t *tokens_categories, int32_t *tokens_attributes, float *confidence,
                            float *image_confidence, float conf_scale, void *stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Graph-captured inference with the early exit decided on the device (conditional graph nodes, CUDA 12.4+).
+ * A forward of N boosted blocks has N - 1 boundaries; boundary i decides whether block i + 1 runs.  The caller
+ *   1. bdetr_exit_graph_create(N - 1, &g, handles): the top-level graph and one IF-node handle per boundary;
+ *   2. captures N + 1 segments on its own: S0 = everything before block 0 plus block 0, Sk = block k (k >= 1),
+ *      E = bdetr_select_exit_predictions.  Each Sk with k < N - 1 ends with bdetr_inverse_tokenize of block k's running
+ *      category prediction and bdetr_early_exit_decide(boundary k, next_block = handles[k]).  A segment must not wait on
+ *      an event recorded in another one, and may contain kernel, memset, memcpy, empty and child-graph nodes only (the
+ *      nodes CUDA allows inside a conditional body);
+ *   3. bdetr_exit_graph_build(g, segments, N + 1) -> child(S0) -> IF(h0){S1} -> ... -> IF(h_{N-2}){S_{N-1}} -> child(E),
+ *      instantiated (the segments are cloned: the caller may destroy its own graphs afterwards);
+ *   4. bdetr_exit_graph_launch(g, stream) per call; bdetr_exit_graph_destroy(g) at the end.
+ * Every handle resets to 0 at launch, so once a boundary exits, no later block runs.
+ * ---------------------------------------------------------------------------------------- */
+#define BDETR_MAX_EXIT_BLOCKS 32
+typedef struct bdetr_exit_graph bdetr_exit_graph;
+int bdetr_exit_graph_create(int n_boundaries, bdetr_exit_graph **g, unsigned long long *handles);
+int bdetr_exit_graph_build(bdetr_exit_graph *g, void *const *segments, int n_segments);
+int bdetr_exit_graph_launch(bdetr_exit_graph *g, void *stream);
+int bdetr_exit_graph_destroy(bdetr_exit_graph *g);
+/* One CTA.  image_conf [B] = the image confidences of the running prediction after block `boundary` (bdetr_inverse_tokenize
+ * with conf_scale = 1 / (boundary + 2)).  Device words: threshold (float32), min_blocks, threshold_set (0 / 1).  Block
+ * boundary + 1 runs when boundary + 1 < min_blocks, or threshold_set == 0, or some image has !(image_conf >= threshold)
+ * (the eager rule: float32 compare, inclusive, a NaN confidence is not confident).  Writes exit_block = boundary when it
+ * exits and n_blocks - 1 otherwise, copies image_conf into conf_out [B], and sets the condition of `next_block` (0 = no
+ * conditional node: the decision is only written). */
+int bdetr_early_exit_decide(int B, int boundary, int n_blocks, const float *image_conf, const float *threshold,
+                            const int32_t *min_blocks, const int32_t *threshold_set, unsigned long long next_block,
+                            int32_t *exit_block, float *conf_out, void *stream);
+/* cums [3 * n_blocks] = the running category [B,Q,C], attribute [B,Q,A] and box [B,Q,4] predictions of block 0, 1, ...;
+ * copies those of block *exit_block (read on the device) into cat / attr / box.  n_blocks <= BDETR_MAX_EXIT_BLOCKS. */
+int bdetr_select_exit_predictions(int n_blocks, int B, int Q, int C, int A, const float *const *cums,
+                                  const int32_t *exit_block, float *cat, float *attr, float *box, void *stream);
 
 /* ------------------------------------------------------------------------------------------
  * Data parallel (SURVEY 8e): the gradient all-reduce, the only collective on the path.  The reference's
