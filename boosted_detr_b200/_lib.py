@@ -78,6 +78,7 @@ PROTOTYPES = {
     "bdetr_attention_block_fwd": (c_int, [I, I, I, I, I, P, P, P, POINTER(AttnParams), F, c_uint32, P, F, P,
                                           POINTER(AttnSaved), P]),
     "bdetr_attention_core_fwd": (c_int, [I, I, I, I, I, P, P, P, P, P, P]),
+    "bdetr_attention_core_bwd": (c_int, [I, I, I, I, I, P, P, P, P, P, P, P, P, P, P, P]),
     "bdetr_attention_block_bwd": (c_int, [I, I, I, I, I, P, P, P, POINTER(AttnParams), F, c_uint32, P,
                                           POINTER(AttnSaved), P, P, P, P, I, POINTER(AttnParams),
                                           POINTER(AttnScratch), P]),

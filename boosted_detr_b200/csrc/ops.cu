@@ -69,6 +69,15 @@ API int bdetr_attention_core_fwd(int B, int H, int Lq, int Lk, int d, const floa
     return launch_attention_fwd(B, H, Lq, Lk, d, qp, kp, vp, o, lse, 0, as_stream(stream));
 }
 
+API int bdetr_attention_core_bwd(int B, int H, int Lq, int Lk, int d, const float *qp, const float *kp, const float *vp,
+                                 const float *o, const float *lse, const float *d_o, float *delta,
+                                 float *d_qp, float *d_kp, float *d_vp, void *stream)
+{
+    BDETR_REQUIRE(qp && kp && vp && o && lse && d_o && delta && d_qp && d_kp && d_vp, BDETR_E_NULL, "null pointer");
+    BDETR_REQUIRE(B > 0 && H > 0 && Lq > 0 && Lk > 0, BDETR_E_BAD_SHAPE, "bad attention shape");
+    return launch_attention_bwd(B, H, Lq, Lk, d, qp, kp, vp, o, lse, d_o, delta, d_qp, d_kp, d_vp, 0, as_stream(stream));
+}
+
 API size_t bdetr_attention_f16_workspace_bytes(int B, int H, int Lq, int Lk, int d)
 {
     if (B <= 0 || H <= 0 || Lq <= 0 || Lk <= 0) return 0;

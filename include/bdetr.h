@@ -46,7 +46,8 @@ typedef enum {
                            * layers hand ws16 over for inference forwards only). */
 
 /* 101: attention at head dim 64 (D/H = 64) besides 32
- * 103: graph-captured inference with the early exit on the device (bdetr_exit_graph_*, bdetr_early_exit_decide) */
+ * 103: graph-captured inference with the early exit on the device (bdetr_exit_graph_*, bdetr_early_exit_decide)
+ * 104: the attention core backward exported on its own (bdetr_attention_core_bwd) */
 int bdetr_version(void);
 const char *bdetr_last_error(void);
 /* Process-wide compute mode used by the dense entry points. */
@@ -218,6 +219,12 @@ int bdetr_attention_block_fwd(int B, int Lq, int Lk, int D, int H,
  * Tensor-core mode runs the tcgen05/TMEM flash kernel; fp32 mode the SIMT kernel. */
 int bdetr_attention_core_fwd(int B, int H, int Lq, int Lk, int d, const float *qp, const float *kp, const float *vp,
                              float *o, float *lse, void *stream);
+/* Backward of bdetr_attention_core_fwd: qp [B,Lq,H*d], kp/vp [B,Lk,H*d], o / d_o [B,H,Lq,d], lse [B,H,Lq] (log2 units,
+ * as the forward writes it); writes delta [B,H,Lq] = sum_d d_o*o, d_qp [B,Lq,H*d], d_kp / d_vp [B,Lk,H*d] (overwritten,
+ * not rounded).  Tensor-core mode: the tcgen05 kernels; fp32 mode: the SIMT kernels.  d = 32 or 64. */
+int bdetr_attention_core_bwd(int B, int H, int Lq, int Lk, int d, const float *qp, const float *kp, const float *vp,
+                             const float *o, const float *lse, const float *d_o, float *delta,
+                             float *d_qp, float *d_kp, float *d_vp, void *stream);
 
 /* fp16-operand attention core (BDETR_MODE_FP16; reference policy: parameters.py:73 `mixed_float16`).  Same contract as
  * bdetr_attention_core_fwd; ws16 = bdetr_attention_f16_workspace_bytes(...) bytes of caller-owned scratch (fp16 copies of

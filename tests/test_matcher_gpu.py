@@ -86,7 +86,13 @@ def _check_assign(cost, n):
     assert (r4c == inv).all()
 
 
-@pytest.mark.parametrize("T,Q", [(20, 100), (100, 300), (7, 7), (33, 32), (64, 65), (100, 100)])
+# (20, 400) general solver, cost staged; (100, 400) general solver, unstaged; (130, 100) more targets than predictions,
+# unstaged; (40, 307) register solver, staged, above 48 KB of dynamic shared memory; (20, 128) / (20, 129) the two
+# register widths
+LSAP_GENERAL = [(20, 400), (100, 400), (130, 100), (40, 307), (20, 128), (20, 129)]
+
+
+@pytest.mark.parametrize("T,Q", [(20, 100), (100, 300), (7, 7), (33, 32), (64, 65), (100, 100)] + LSAP_GENERAL)
 def test_lsap_bitexact_random(T, Q):
     rng = np.random.default_rng(T * 7 + Q)
     B = 48
@@ -96,7 +102,7 @@ def test_lsap_bitexact_random(T, Q):
     _check_assign(rng.random((B, T, Q)) * 1000.0 + 3.0, n)
 
 
-@pytest.mark.parametrize("T,Q", [(20, 100), (12, 12), (40, 50)])
+@pytest.mark.parametrize("T,Q", [(20, 100), (12, 12), (40, 50)] + LSAP_GENERAL)
 def test_lsap_bitexact_ties(T, Q):
     rng = np.random.default_rng(T + Q)
     B = 64
@@ -122,27 +128,55 @@ def test_lsap_more_targets_than_predictions():
     _check_assign(np.round(rng.random((B, T, Q)) * 4) / 4, n)
 
 
-def test_lsap_error_status():
+def _check_error_status(T, Q):
+    """Per-image status and results next to invalid and infeasible images, with status words, index outputs and mask
+    that start out holding garbage, and one image with more objects than target rows (it behaves like cost[b, :n])."""
     from boosted_detr_b200 import _lib
+    from boosted_detr_b200.device import ptr, stream_ptr
     from boosted_detr_b200.losses_and_metrics import MatchingAssignment, raise_for_status
     rng = np.random.default_rng(9)
-    B, T, Q = 5, 6, 9
+    B = 6
     cost = rng.random((B, T, Q)).astype(np.float32)
     n = np.full(B, T, np.int32)
     n[3] = 2
+    n[5] = T + 3
     cost[1, 2, 3] = np.nan
     cost[2, 0, 0] = -np.inf
     cost[3, 4, 4] = np.nan            # beyond num_objects: ignored like cost[i,:n_i,:]
     cost[4, 1, :] = np.inf            # infeasible row
-    c4r, r4c, mask, assigned, status = _gpu_assign(cost, n)
-    assert list(status) == [0, _lib.BDETR_E_INVALID_COST, _lib.BDETR_E_INVALID_COST, 0, _lib.BDETR_E_INFEASIBLE]
-    assert (c4r[1] == -1).all() and (c4r[4] == -1).all()
-    r, c = linear_sum_assignment(cost[0])
-    assert (c4r[0] == c).all()
+    dc, dn = _dev(cost, n)
+    c4r = torch.full((B, T), 7, dtype=torch.int32, device="cuda")
+    r4c = torch.full((B, Q), 7, dtype=torch.int32, device="cuda")
+    mask = torch.full((B, T, Q), 7.0, device="cuda")
+    assigned = torch.full((B, Q), 7.0, device="cuda")
+    status = torch.full((B,), 12345, dtype=torch.int32, device="cuda")
+    _lib.call("bdetr_lsap_assign", B, T, Q, ptr(dc), ptr(dn), ptr(c4r), ptr(r4c), ptr(mask), ptr(assigned), ptr(status),
+              stream_ptr())
+    c4r, r4c, mask, assigned, status = (t.cpu().numpy() for t in (c4r, r4c, mask, assigned, status))
+    assert list(status) == [0, _lib.BDETR_E_INVALID_COST, _lib.BDETR_E_INVALID_COST, 0, _lib.BDETR_E_INFEASIBLE, 0]
+    assert (c4r[1] == -1).all() and (c4r[4] == -1).all() and (r4c[1] == -1).all() and (r4c[4] == -1).all()
+    for b in (0, 3, 5):
+        r, c = linear_sum_assignment(cost[b, :n[b]])
+        exp_c4r, exp_r4c, exp_mask = np.full(T, -1), np.full(Q, -1), np.zeros((T, Q), np.float32)
+        exp_c4r[r], exp_r4c[c], exp_mask[r, c] = c, r, 1.0
+        assert (c4r[b] == exp_c4r).all() and (r4c[b] == exp_r4c).all(), b
+        assert (mask[b] == exp_mask).all() and (assigned[b] == exp_mask.max(axis=0)).all(), b
     with pytest.raises(ValueError, match="invalid numeric"):
         MatchingAssignment()(*_dev(cost, n))
     with pytest.raises(ValueError, match="infeasible"):
         raise_for_status(torch.tensor([0, _lib.BDETR_E_INFEASIBLE]))
+
+
+def test_lsap_error_status():
+    """Validation fused into the register solver's staging copy."""
+    _check_error_status(6, 9)
+
+
+@pytest.mark.parametrize("T,Q", [(20, 400), (100, 300)])
+def test_lsap_error_status_separate_validate(T, Q):
+    """The general solver (20, 400) and the register solver on an unstaged cost (100, 300), both behind the separate
+    validate kernel and a memset of the status words."""
+    _check_error_status(T, Q)
 
 
 def test_end_to_end_assignment_on_gpu_cost():
@@ -176,12 +210,42 @@ def test_step0_identical_predictions():
     _check_assign(cost, tr[3])
 
 
-@pytest.mark.parametrize("B,T,Q,C,A,w_attr", [(2, 20, 100, 82, 3, 1.0), (3, 20, 100, 48, 296, 1.0), (4, 9, 17, 6, 5, 0.0)])
+def test_cost_matrix_fwd_equals_prepared_path():
+    """bdetr_cost_matrix_fwd -- the prepared path on a library-owned, grow-only scratch buffer -- gives the bits of
+    bdetr_cost_targets_prepare + bdetr_cost_matrix_prepared.  The second, larger shape makes the buffer grow."""
+    from boosted_detr_b200 import _lib
+    from boosted_detr_b200.device import ptr, stream_ptr
+    from boosted_detr_b200.losses_and_metrics import pairwise_cost
+    for B, T, Q, C, A in [(2, 5, 7, 5, 2), (8, 100, 300, 1205, 3)]:
+        rng = np.random.default_rng(T + C)
+        tr = _dev(*synth_targets(rng, B, T, C, A, attr_p=0.05)[:3])
+        pr = _dev(*synth_preds(rng, B, Q, C, A))
+        want = pairwise_cost(tr, pr, W[0], W[1], W[2]).cpu().numpy()
+        got = torch.full((B, T, Q), float("nan"), device="cuda")
+        _lib.call("bdetr_cost_matrix_fwd", B, T, Q, C, A, *(ptr(t) for t in tr), *(ptr(t) for t in pr), W[0], W[1], W[2],
+                  ptr(got), stream_ptr())
+        got = got.cpu().numpy()
+        assert np.isfinite(want).all()
+        assert np.array_equal(got.view(np.int32), want.view(np.int32)), (B, T, Q, C, A)
+
+
+# (2, 32, 100, 82, 3): the last T of the warp-per-row form; T > 32 runs one thread per row, with the attribute term
+# inline for A <= 8 ((2, 100, 300, 82, 3) is BASELINE config 4) and a warp per row above ((2, 33, 65, 33, 9), and
+# (2, 40, 100, 48, 296) at the Fashionpedia A); (1, 300, 300, 82, 8): more rows than the 256 threads of the CTA
+@pytest.mark.parametrize("B,T,Q,C,A,w_attr", [(2, 20, 100, 82, 3, 1.0), (3, 20, 100, 48, 296, 1.0), (4, 9, 17, 6, 5, 0.0),
+                                              (2, 32, 100, 82, 3, 1.0), (2, 100, 300, 82, 3, 1.0), (2, 100, 300, 82, 3, 0.0),
+                                              (2, 33, 65, 33, 9, 1.0), (2, 40, 100, 48, 296, 1.0), (1, 300, 300, 82, 8, 1.0)])
 def test_matched_loss_and_gradient_vs_oracle(B, T, Q, C, A, w_attr):
+    """Matched losses, IoU metric and gradients against the fp64 oracle given the GPU's assignment.  Caught at T = 32: the
+    accumulation check compared with the fp64 gradient element by element at rtol 1e-4, which fp32 arithmetic itself
+    misses where box terms cancel (the fp32 oracle by 3.7e-4); it now compares with the first call's own gradient."""
     from oracle import reference_path as R
     from boosted_detr_b200.losses_and_metrics import MatchingLoss
     rng = np.random.default_rng(17 + B)
     tr = synth_targets(rng, B, T, C, A, attr_p=0.05)
+    if T >= 32:         # the last image with every target row live, so that the last row (t = T - 1) is matched
+        for x, f in zip(tr, synth_targets(rng, 1, T, C, A, attr_p=0.05, min_n=T)):
+            x[-1] = f[0]
     pr = synth_preds(rng, B, Q, C, A, k_sum=2)
     pr[0][0, :5, 0] = 1.2          # saturate safe_clip on a few entries (zero gradient there)
     pr[0][0, 5:9, 0] = 0.0001
@@ -199,9 +263,15 @@ def test_matched_loss_and_gradient_vs_oracle(B, T, Q, C, A, w_attr):
     y_true = [torch.tensor(tr[0], dtype=dt), torch.tensor(tr[1], dtype=dt), torch.tensor(tr[2], dtype=dt), tr[3]]
     y_pred = [torch.tensor(p, dtype=dt, requires_grad=True) for p in pr]
     ref_losses, ref_iou, ref_mask, _ = R.matching_loss(y_true, y_pred, w, mask=torch.tensor(mask, dtype=dt))
-    # and the oracle's own assignment must agree with the GPU's on this data
-    _, _, own_mask, _ = R.matching_loss(y_true, [p.detach() for p in y_pred], w)
-    assert (own_mask.numpy() == mask).all()
+    # and the oracle's own assignment must agree with the GPU's on this data -- or, where the GPU's fp32 cost and the
+    # oracle's differ in their last bits at a near-tie (possible at T >= 100), be just as optimal under the fp64 cost
+    _, _, own_mask, cost64 = R.matching_loss(y_true, [p.detach() for p in y_pred], w)
+    own_mask = own_mask.numpy()
+    if not (own_mask == mask).all():
+        cost64 = cost64.numpy()
+        tot_gpu, tot_own = (cost64 * mask).sum((1, 2)), (cost64 * own_mask).sum((1, 2))
+        print(f"assignments differ at a near-tie: optimal totals {tot_own} (oracle) vs {tot_gpu} (GPU)")
+        assert np.abs(tot_gpu - tot_own).max() <= 1e-6 * np.abs(tot_own).max()
     for k, name in enumerate(["total", "cat", "attr", "box", "exist"]):
         g = losses[k].cpu().numpy().astype(np.float64)
         r = ref_losses[k].detach().numpy()
@@ -220,9 +290,11 @@ def test_matched_loss_and_gradient_vs_oracle(B, T, Q, C, A, w_attr):
         rel = np.abs(g - r).max() / max(np.abs(r).max(), 1e-30)
         print(f"{name}: rel {rel:.2e} (max |ref| {np.abs(r).max():.3e})")
         assert rel < 1e-5, name
-    # accumulate semantics + gscale
+    # accumulate semantics + gscale: a second call with gscale 0.5 adds half of the first call's gradient
+    first = [t.cpu().numpy() for t in d]
     ml.backward(ctx, d[0], d[1], d[2], gscale=0.5)
-    assert np.allclose(d[2].cpu().numpy(), 1.5 * y_pred[2].grad.numpy(), rtol=1e-4, atol=1e-7)
+    for got, g1, name in zip(d, first, ["d_cat", "d_attr", "d_box"]):
+        assert np.allclose(got.cpu().numpy(), 1.5 * g1, rtol=1e-6, atol=0), name
 
 
 def test_matcher_stress_full_size_properties():

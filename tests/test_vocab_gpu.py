@@ -109,14 +109,18 @@ def test_heads_fused_wide_identical_rows_stay_identical(tc_mode):
 
 
 # ---- 2. cost matrix, assignment, matched loss ------------------------------------------------------------------------
-@pytest.mark.parametrize("B,T,Q,C,A,multi_hot", [(2, 20, 100, 367, 3, 0), (2, 20, 100, 1205, 3, 0), (2, 100, 300, 1205, 3, 0),
-                                                 (2, 20, 100, 2048, 3, 0), (2, 20, 100, 1205, 296, 0),
-                                                 (2, 20, 100, 1205, 3, 4)])
-def test_cost_matrix_wide_vs_oracle(B, T, Q, C, A, multi_hot):
+_WIDE = [(2, 20, 100, 367, 3, 0), (2, 20, 100, 1205, 3, 0), (2, 100, 300, 1205, 3, 0), (2, 20, 100, 2048, 3, 0),
+         (2, 20, 100, 1205, 296, 0), (2, 20, 100, 1205, 3, 4)]
+
+
+@pytest.mark.parametrize("B,T,Q,C,A,multi_hot,w_attr",
+                         [pytest.param(*c, 1.0, id="-".join(map(str, c))) for c in _WIDE]
+                         + [(2, 20, 100, 1205, 3, 0, 0.0), (2, 100, 300, 2048, 3, 0, 0.0)])
+def test_cost_matrix_wide_vs_oracle(B, T, Q, C, A, multi_hot, w_attr):
     """Costs of the wide digest + gather cost kernels within 3 ulp of the fp32 oracle, built one image at a time; the
     assignment on the GPU cost bit-exact against scipy.  multi_hot: that many target rows per image carry five
     classes each, so the image has more class slots than target rows (the slots past the staged ones are read from
-    global memory)."""
+    global memory).  w_attr = 0: the gather kernel without the attribute term."""
     from boosted_detr_b200.losses_and_metrics import pairwise_cost
     rng = np.random.default_rng(C + T + A + multi_hot)
     tr = synth_targets(rng, B, T, C, A, attr_p=0.05)
@@ -125,19 +129,20 @@ def test_cost_matrix_wide_vs_oracle(B, T, Q, C, A, multi_hot):
             for t in range(min(multi_hot, int(tr[3][b]))):
                 tr[0][b, t, rng.choice(np.arange(2, C), 5, replace=False)] = 1.0
     pr = synth_preds(rng, B, Q, C, A)
-    got = pairwise_cost(_dev(*tr[:3]), _dev(*pr), W[0], W[1], W[2]).cpu().numpy()
+    w = (W[0], W[1], w_attr, W[3])
+    got = pairwise_cost(_dev(*tr[:3]), _dev(*pr), w[0], w[1], w[2]).cpu().numpy()
     assert np.isfinite(got).all()
     worst = 0
     for b in range(B):
         one = lambda arrs: [a[b:b + 1] for a in arrs]
         trb = one(tr[:3]) + [tr[3][b:b + 1]]
-        ref32 = _oracle_cost(trb, one(pr), W, torch.float32)[0]
+        ref32 = _oracle_cost(trb, one(pr), w, torch.float32)[0]
         if multi_hot:       # a sum over several classes: the oracle sums in its own order
-            ref64 = _oracle_cost(trb, one(pr), W, torch.float64)[0]
+            ref64 = _oracle_cost(trb, one(pr), w, torch.float64)[0]
             assert np.abs(got[b] - ref64).max() / np.abs(ref64).max() < 1e-5
         else:
             worst = max(worst, int(_ulp_diff(got[b], ref32).max()))
-    print(f"cost[{B},{T},{Q}] C={C} A={A}: max ulp vs fp32 oracle {worst}")
+    print(f"cost[{B},{T},{Q}] C={C} A={A} w_attr={w_attr}: max ulp vs fp32 oracle {worst}")
     assert worst <= 3
     _check_assign(got, tr[3])
 
