@@ -113,6 +113,11 @@ PROTOTYPES = {
     "bdetr_exit_graph_destroy": (c_int, [P]),
     "bdetr_early_exit_decide": (c_int, [I, I, I, P, P, P, P, c_ulonglong, P, P, P]),
     "bdetr_select_exit_predictions": (c_int, [I, I, I, I, I, POINTER(c_void_p), P, P, P, P, P]),
+    "bdetr_image_exit_state_bytes": (c_size_t, [I, I]),
+    "bdetr_image_exit_plan": (c_int, [I, I, I, I, I, P, P, P, P, c_ulonglong, P, P]),
+    "bdetr_image_exit_compact": (c_int, [I, I, I, I, I, I, I, c_longlong, P, POINTER(PTR3), P, POINTER(PTR3), POINTER(PTR3), P, P]),
+    "bdetr_switch_graph_create": (c_int, [I, I, POINTER(c_void_p), POINTER(c_ulonglong)]),
+    "bdetr_switch_graph_build": (c_int, [P, POINTER(c_void_p), I]),
     "bdetr_comm_unique_id": (c_int, [P]),
     "bdetr_comm_init": (c_int, [POINTER(c_void_p), I, I, P]),
     "bdetr_comm_destroy": (c_int, [P]),

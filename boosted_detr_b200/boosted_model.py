@@ -13,6 +13,7 @@ train_step / test_step (which, as in the reference :269-270, also trains), per-b
 """
 from __future__ import annotations
 
+import ctypes
 import os
 import re
 
@@ -85,6 +86,12 @@ class BoostedDETR:
         self.early_exit_threshold = None
         self.early_exit_min_blocks = 1
         self.last_exit_block = None
+        # Per-image early exit (opt-in, needs a threshold and N >= 2): each image leaves at its own first confident boundary
+        # and the blocks after it run without it (`_forward_per_image`).  After such a call: last_exit_blocks int32 [B],
+        # last_image_confidence [B] (at the exit boundary, or the last boundary checked; NaN if none was) and
+        # last_active_counts int32 [N] (images that ran each block, riders included).
+        self.early_exit_per_image = False
+        self.last_exit_blocks = self.last_active_counts = None
         self._exit_capture = None         # set by graph.GraphedInference while it captures the forward in segments
         self.step_count = 0
         self.num_replicas = 1
@@ -398,6 +405,108 @@ class BoostedDETR:
         self._exit_capture.boundary(i, cums, streams)
         return False
 
+    # -- per-image early exit ---------------------------------------------------------------------
+    def _exit_words(self):
+        """Device words the plan kernel reads: threshold (float32; eager compares float32 confidences with it in float32),
+        [min_blocks, threshold set].  Refilled on the current stream when the settings changed, never inside a capture."""
+        if getattr(self, "_exit_dev", None) is None:
+            self._exit_dev = (torch.zeros(1, dtype=torch.float32, device=require_cuda()),
+                              torch.zeros(2, dtype=torch.int32, device=require_cuda()))
+            self._exit_dev_words = None
+        words = (float(np.float32(self.early_exit_threshold)), int(self.early_exit_min_blocks))
+        if words != self._exit_dev_words and not torch.cuda.is_current_stream_capturing():
+            self._exit_dev[0].fill_(words[0])
+            self._exit_dev[1][0:1].fill_(words[1])
+            self._exit_dev[1][1:2].fill_(1)
+            self._exit_dev_words = words
+        return self._exit_dev
+
+    def _per_image_begin(self, feats):
+        """Prologue of the per-image forward at the full batch B, and what it carries across the boundaries: the gather
+        buffers of x and of the three running predictions (two sets, boundary i writes set i % 2), the outputs and the
+        plan state.  The path chosen at B is kept for the whole call; on the fused path the batch never drops below
+        k_min = the fewest images that fill one 128-row GEMM tile (`_use_fused`)."""
+        B, R, Cc, D = feats.shape
+        N, Q, C, A = self.num_decoder_blocks, self.num_object_preds, self.num_categories, self.num_attributes
+        L = R * Cc
+        if self._use_fused(feats):
+            st = self._fused_prologue(feats, None, False, False, None, 0.0)
+            st.update(fused=True, streams=[st["pre_s"], *st["bstreams"]], k_min=max(-(-128 // L), -(-128 // Q)))
+        else:
+            st = self._layer_prologue(feats, None, False)
+            st.update(fused=False, streams=list(st["aux"]), k_min=1)
+        nbytes = _lib.load().bdetr_image_exit_state_bytes(B, N)
+        st.update(B=B, xp=[empty(B, R, Cc, D) for _ in range(2)], cp=[[empty(B, Q, n) for n in (C, A, 4)] for _ in range(2)],
+                  out=[empty(B, Q, n) for n in (C, A, 4)], conf_q=empty(B, Q), iconf=empty(B), words=self._exit_words(),
+                  state=torch.empty(nbytes // 4, dtype=torch.int32, device=feats.device))
+        return st
+
+    def _per_image_block(self, st, i, k, switch=0):
+        """Block i at batch k (block 0: the prologue's input; later blocks: the first k rows of the gather buffers),
+        every stream joined into the caller's, then boundary i: the image confidences of the k running slots, the plan
+        (`switch` = the graph's SWITCH handle for block i + 1, 0 in eager calls) and the compaction.  After the last
+        block the compaction writes every remaining image out instead."""
+        N, B = self.num_decoder_blocks, st["B"]
+        if i == 0:
+            x, cums = st["x"], None
+        else:
+            x, cums = st["xp"][(i - 1) & 1][:k], [c[:k] for c in st["cp"][(i - 1) & 1]]
+        main = st["main"]
+        if st["fused"]:
+            x, cums, _ = self._fused_block(st, i, x, cums)
+            st["heads_ev"], st["pre_ev"] = None, [None] * N     # joined below: later blocks need no event of this one
+        else:
+            x, cums = self._layer_block(st, i, x, cums)
+        capturing = torch.cuda.is_current_stream_capturing()
+        for s in st["streams"]:
+            with torch.cuda.stream(s):
+                forked = not capturing or torch.cuda.is_current_stream_capturing()   # (a body forks only the streams it uses)
+            if forked:
+                main.wait_stream(s)
+        st["blocks"].clear()                                 # no block context outlives its block
+        _, Q, C = cums[0].shape
+        A = cums[1].shape[-1]
+        cin, out = _lib.PTR3(*[c.data_ptr() for c in cums]), _lib.PTR3(*[o.data_ptr() for o in st["out"]])
+        state = ptr(st["state"])
+        if i == N - 1:
+            _lib.call("bdetr_image_exit_compact", B, N, i, k, Q, C, A, x[0].numel(), None, ctypes.byref(cin), None, None,
+                      ctypes.byref(out), state, stream_ptr())
+            return
+        _lib.call("bdetr_inverse_tokenize", k, Q, C, A, ptr(cums[0]), None, None, None, ptr(st["conf_q"]), ptr(st["iconf"]),
+                  1.0 / (i + 2), stream_ptr())
+        thr, ints = st["words"]
+        _lib.call("bdetr_image_exit_plan", B, N, st["k_min"], i, k, ptr(st["iconf"]), ptr(thr), ptr(ints[0:1]), ptr(ints[1:2]),
+                  switch, state, stream_ptr())
+        cout = _lib.PTR3(*[c.data_ptr() for c in st["cp"][i & 1]])
+        _lib.call("bdetr_image_exit_compact", B, N, i, k, Q, C, A, x[0].numel(), ptr(x), ctypes.byref(cin),
+                  ptr(st["xp"][i & 1]), ctypes.byref(cout), ctypes.byref(out), state, stream_ptr())
+
+    def _forward_per_image(self, feats):
+        """Inference with the per-image early exit.  After each boundary one small D2H of the plan's head words (the
+        number of images that run the next block, the per-block counts, exit blocks and confidences) and one
+        synchronisation -- the per-batch exit also syncs once per boundary -- then the next block is issued at that size."""
+        N = self.num_decoder_blocks
+        st = self._per_image_begin(feats)
+        B = st["B"]
+        head = 1 + N + 2 * B
+        if getattr(self, "_pi_host", None) is None or self._pi_host.numel() != head:
+            self._pi_host = torch.empty(head, dtype=torch.int32).pin_memory()
+        k = B
+        for i in range(N):
+            self._per_image_block(st, i, k)
+            self.last_exit_block = i
+            if i == N - 1:
+                break
+            self._pi_host.copy_(st["state"][:head], non_blocking=True)
+            torch.cuda.current_stream().synchronize()
+            k = int(self._pi_host[0])
+            if k == 0:
+                break
+        h = self._pi_host.clone()
+        self.last_active_counts, self.last_exit_blocks = h[1:1 + N], h[1 + N:1 + N + B]
+        self.last_image_confidence = h[1 + N + B:].view(torch.float32)
+        return st["out"], {"blocks": [], "loss": [], "y_true": None}
+
     # -- fused tensor-core path -------------------------------------------------------------------
     def _use_fused(self, feats):
         """Tensor-core mode, model width 256, every layer already built (the very first call builds the layers lazily
@@ -433,16 +542,41 @@ class BoostedDETR:
 
     def _forward_fused_on(self, feats, y_true, training, use_dropout, seed_dev, rate):
         N = self.num_decoder_blocks
+        st = self._fused_prologue(feats, y_true, training, use_dropout, seed_dev, rate)
+        main, pre_s, bstreams = st["main"], st["pre_s"], st["bstreams"]
+        x, cums = st["x"], None
+        for i in range(N):
+            x, cums, bs = self._fused_block(st, i, x, cums)
+            with torch.cuda.stream(bs):
+                self.last_exit_block = i
+                if not training:
+                    if self._exit_boundary(i, cums, [main, pre_s, *bstreams]):
+                        break
+                    if self._exit_capture is not None:
+                        # a new graph segment has begun behind a join of every stream: events recorded in the previous
+                        # segments cannot be waited on, and the join already orders everything after them
+                        st["heads_ev"], st["pre_ev"] = None, [None] * N
+        for bs in bstreams:
+            main.wait_stream(bs)
+        main.wait_stream(pre_s)
+        if training:
+            main.wait_stream(st["side"])
+        self._mark("fwd joined (main)")
+        return cums, {"blocks": st["blocks"], "loss": st["loss_ctxs"], "y_true": y_true, "fused": True}
+
+    def _fused_prologue(self, feats, y_true, training, use_dropout, seed_dev, rate):
+        """Everything of `_forward_fused_on` before block 0, at the full batch: the rounded input, the target digest, and
+        the weight-only work (positional tables, tiled queries, hoisted decoder self-attention) on the aux2 stream."""
+        N = self.num_decoder_blocks
         main = torch.cuda.current_stream()
         side = self._side_stream() if training else None
         aux = self._aux_streams()
-        dec_s, pre_s = aux[3], aux[2]
+        pre_s = aux[2]
         self.refresh_shadow()
         x = torch.empty_like(feats)                        # the block input feeds tcgen05 GEMMs: round it too
         _lib.call("bdetr_round_tf32", feats.numel(), ptr(feats), ptr(x), stream_ptr())
         B, R, Cc, D = feats.shape
-        L, Q = R * Cc, self.num_object_preds
-        prepared, loss_streams = None, None
+        prepared = None
         if training:
             side.wait_stream(main)
             with torch.cuda.stream(side):
@@ -474,54 +608,50 @@ class BoostedDETR:
                 ev = torch.cuda.Event()
                 ev.record(pre_s)
                 pre_ev.append(ev)
-        cums = None
-        blocks, loss_ctxs = [], []
         # decoder i / heads i / matching i hang off encoder i's output only (plus the running prediction of block i-1):
         # every block gets its own side stream, so decoder i overlaps heads i-1 and the matchings
-        bstreams = self._block_streams(N)
-        heads_ev = None
-        for i in range(N):
-            keys = self._keys(i) if use_dropout else None
-            enc, dec_l = self.EncoderTransformerBlocks[i], self.DecoderBlocks[i]
-            dkeys = keys["dec"] if keys else (0, 0, 0)
-            if pre_ev[i] is not None:
-                main.wait_event(pre_ev[i])
-            (x, pos), c_enc = enc.forward([x], training, keys["enc"] if keys else None, seed_dev, tabs=tabs[i][:2])
-            self._mark(f"fwd enc{i} done (main)")
-            bs = bstreams[i]
-            bs.wait_stream(main)
-            with torch.cuda.stream(bs):
-                fold = make_fold(pos=pos.view(L, D), tab_k=tabs[i][2], pos_tc=enc.pos_tc())
-                dec_in = dec0 if i == 0 else pre_self[i][0]
-                dec, c_dec = dec_l.forward_fused(x.view(B, L, D), fold, dec_in, training, dkeys, seed_dev)
-                self._mark(f"fwd dec{i} done (dec)")
-                mult = 2.0 if i == 0 else 1.0                 # block 0 is counted twice (reference :222-229)
-                heads = (self.CategoryBlocks[i], self.AttributeBlocks[i], self.BoxBlocks[i])
-                if heads_ev is not None:
-                    bs.wait_event(heads_ev)                   # the running prediction of block i-1
-                cums, c_heads = heads_forward_fused(heads, dec, training, cums, mult)
-                heads_ev = torch.cuda.Event()
-                heads_ev.record(bs)
-                self._mark(f"fwd heads{i} done (dec)")
-                blocks.append({"enc": c_enc, "dec": c_dec, "self": None if i == 0 else pre_self[i][1], "heads": c_heads, "dec0": dec0})
-                if training:
-                    loss_ctxs.append(self.loss_fn.forward(y_true, cums, prepared))
-                    self._mark(f"fwd loss{i} done (side)")
-                self.last_exit_block = i
-                if not training:
-                    if self._exit_boundary(i, cums, [main, pre_s, *bstreams]):
-                        break
-                    if self._exit_capture is not None:
-                        # a new graph segment has begun behind a join of every stream: events recorded in the previous
-                        # segments cannot be waited on, and the join already orders everything after them
-                        heads_ev, pre_ev = None, [None] * N
-        for bs in bstreams:
-            main.wait_stream(bs)
-        main.wait_stream(pre_s)
-        if training:
-            main.wait_stream(side)
-        self._mark("fwd joined (main)")
-        return cums, {"blocks": blocks, "loss": loss_ctxs, "y_true": y_true, "fused": True}
+        return {"main": main, "side": side, "pre_s": pre_s, "bstreams": self._block_streams(N), "x": x, "B": B, "L": R * Cc,
+                "D": D, "training": training, "use_dropout": use_dropout, "seed_dev": seed_dev, "y_true": y_true,
+                "prepared": prepared, "tabs": tabs, "pre_self": pre_self, "pre_ev": pre_ev, "dec0": dec0, "heads_ev": None,
+                "blocks": [], "loss_ctxs": []}
+
+    def _fused_block(self, st, i, x, cums):
+        """Boosted block i of the fused path on x [k, R, Cc, D] (k <= the prologue's batch: the tiled queries and the hoisted
+        self-attention are the same for every image, so their first k rows serve).  Returns (encoder output, running
+        predictions, the block's stream, on which they are final)."""
+        training, use_dropout, seed_dev = st["training"], st["use_dropout"], st["seed_dev"]
+        main, L, D = st["main"], st["L"], st["D"]
+        k = x.shape[0]
+        keys = self._keys(i) if use_dropout else None
+        enc, dec_l = self.EncoderTransformerBlocks[i], self.DecoderBlocks[i]
+        dkeys = keys["dec"] if keys else (0, 0, 0)
+        if st["pre_ev"][i] is not None:
+            main.wait_event(st["pre_ev"][i])
+        (x, pos), c_enc = enc.forward([x], training, keys["enc"] if keys else None, seed_dev, tabs=st["tabs"][i][:2])
+        self._mark(f"fwd enc{i} done (main)")
+        bs = st["bstreams"][i]
+        bs.wait_stream(main)
+        with torch.cuda.stream(bs):
+            fold = make_fold(pos=pos.view(L, D), tab_k=st["tabs"][i][2], pos_tc=enc.pos_tc())
+            dec_in = st["dec0"] if i == 0 else st["pre_self"][i][0]
+            if k != dec_in.shape[0]:
+                dec_in = dec_in[:k]
+            dec, c_dec = dec_l.forward_fused(x.view(k, L, D), fold, dec_in, training, dkeys, seed_dev)
+            self._mark(f"fwd dec{i} done (dec)")
+            mult = 2.0 if i == 0 else 1.0                 # block 0 is counted twice (reference :222-229)
+            heads = (self.CategoryBlocks[i], self.AttributeBlocks[i], self.BoxBlocks[i])
+            if st["heads_ev"] is not None:
+                bs.wait_event(st["heads_ev"])             # the running prediction of block i-1
+            cums, c_heads = heads_forward_fused(heads, dec, training, cums, mult)
+            st["heads_ev"] = torch.cuda.Event()
+            st["heads_ev"].record(bs)
+            self._mark(f"fwd heads{i} done (dec)")
+            st["blocks"].append({"enc": c_enc, "dec": c_dec, "self": None if i == 0 else st["pre_self"][i][1], "heads": c_heads,
+                                 "dec0": st["dec0"]})
+            if training:
+                st["loss_ctxs"].append(self.loss_fn.forward(st["y_true"], cums, st["prepared"]))
+                self._mark(f"fwd loss{i} done (side)")
+        return x, cums, bs
 
     def _trainable_flags(self):
         N = self.num_decoder_blocks
@@ -696,8 +826,37 @@ class BoostedDETR:
             aux2     decoder self-attention of block i >= 1 (queries only: no dependency on the image at all)
             side     cost matrix -> per-image assignment -> matched loss of block i (forked from dec)
         and everything is joined into main before returning."""
+        if not training and self.early_exit_per_image and self.early_exit_threshold is not None and self.num_decoder_blocks >= 2:
+            return self._forward_per_image(feats)
         if self._use_fused(feats):
             return self._forward_fused(feats, y_true, training)
+        N = self.num_decoder_blocks
+        st = self._layer_prologue(feats, y_true, training)
+        main, aux, dec_s = st["main"], st["aux"], st["dec_s"]
+        x, cums = st["x"], None
+        for i in range(N):
+            x, cums = self._layer_block(st, i, x, cums)
+            with torch.cuda.stream(dec_s):
+                self.last_exit_block = i
+                if not training and self._exit_boundary(i, cums, [main, *aux]):
+                    break
+                if training:
+                    ls = st["loss_streams"][i]
+                    ls.wait_stream(dec_s)
+                    with torch.cuda.stream(ls):
+                        st["loss_ctxs"].append(self.loss_fn.forward(y_true, cums, st["prepared"]))
+                        self._mark(f"fwd loss{i} done (side)")
+        main.wait_stream(dec_s)
+        main.wait_stream(aux[2])
+        if training:
+            main.wait_stream(st["side"])
+            for ls in st["loss_streams"]:
+                main.wait_stream(ls)
+        self._mark("fwd joined (main)")
+        return cums, {"blocks": st["blocks"], "loss": st["loss_ctxs"], "y_true": y_true}
+
+    def _layer_prologue(self, feats, y_true, training):
+        """Everything of the layer-level `forward` before block 0: the (rounded) input and the target digest."""
         N = self.num_decoder_blocks
         use_dropout = training and self.dropout_seed is not None
         if use_dropout and not torch.cuda.is_current_stream_capturing():
@@ -707,14 +866,11 @@ class BoostedDETR:
         main = torch.cuda.current_stream()
         side = self._side_stream() if training else None
         aux = self._aux_streams()
-        dec_s = aux[3]
         if self.tensor_core_mode():
             self.refresh_shadow()
             x = torch.empty_like(feats)                        # the block input feeds tcgen05 GEMMs: round it too
             _lib.call("bdetr_round_tf32", feats.numel(), ptr(feats), ptr(x), stream_ptr())
-        cums = None
-        blocks, loss_ctxs = [], []
-        prepared = None
+        prepared, loss_streams = None, None
         if training:                                           # one target batch, N matchings: digest the targets once
             side.wait_stream(main)
             with torch.cuda.stream(side):
@@ -725,68 +881,58 @@ class BoostedDETR:
             loss_streams = self._loss_streams(N)
             for ls in loss_streams:
                 ls.wait_stream(side)
-        for i in range(N):
-            keys = self._keys(i) if use_dropout else None
-            enc = self.EncoderTransformerBlocks[i]
-            for blk in enc.EncoderBlocks:
-                blk.SelfAttentionBlock.rate = blk.FeedForwardBlock.rate = 0.1 if use_dropout else 0.0
-            dec_l = self.DecoderBlocks[i]
-            for nm in ("SelfAttentionBlock", "JointAttentionBlock", "FeedForwardBlock"):
-                if hasattr(dec_l, nm):
-                    getattr(dec_l, nm).rate = 0.1 if use_dropout else 0.0
-            dkeys = keys["dec"] if keys else (0, 0, 0)
-            pre_self, dec0 = None, None
-            # (not on the very first call: layers build lazily in execution order, and the weight-initialisation
-            # order -- hence the seeded initial weights -- must not depend on this scheduling choice)
-            if hasattr(dec_l, "SelfAttentionBlock") and dec_l.SelfAttentionBlock.built:
-                aux[2].wait_stream(main)
-                with torch.cuda.stream(aux[2]):
-                    dec0 = self.DecoderPrep.tile_queries(x.shape[0], like=x)
-                    pre_self = dec_l.SelfAttentionBlock.forward([dec0, dec0, dec0], training, dkeys[0], seed_dev)
-            (x, pos), c_enc = enc.forward([x], training, keys["enc"] if keys else None, seed_dev)
-            self._mark(f"fwd enc{i} done (main)")
-            dec_s.wait_stream(main)
-            with torch.cuda.stream(dec_s):
-                prep_out, c_prep = self.DecoderPrep.forward([x, pos], training, dec=dec0)
-                if pre_self is not None:
-                    dec_s.wait_stream(aux[2])
-                dec, c_dec = dec_l.forward(list(prep_out), training, dkeys, pre_self=pre_self, seed_dev=seed_dev)
-                self._mark(f"fwd dec{i} done (dec)")
-                mult = 2.0 if i == 0 else 1.0                 # block 0 is counted twice (reference :222-229)
-                if cums is not None and training:
-                    cums = [c.clone() for c in cums]          # each block's loss keeps its own running prediction
-                heads = (self.CategoryBlocks[i], self.AttributeBlocks[i], self.BoxBlocks[i])
-                c_heads, new_cums = [], []
-                for h, head in enumerate(heads):              # three independent chains: one stream each
-                    st = dec_s if h == 0 else aux[h - 1]
-                    if st is not dec_s:
-                        st.wait_stream(dec_s)
-                    with torch.cuda.stream(st):
-                        _, c = head.forward([dec], training, cum=None if cums is None else cums[h], mult=mult)
-                    c_heads.append(c)
-                    new_cums.append(c["cum"])
-                dec_s.wait_stream(aux[0])
-                dec_s.wait_stream(aux[1])
-                self._mark(f"fwd heads{i} done (dec)")
-                cums = new_cums
-                blocks.append({"enc": c_enc, "prep": c_prep, "dec": c_dec, "heads": c_heads})
-                self.last_exit_block = i
-                if not training and self._exit_boundary(i, cums, [main, *aux]):
-                    break
-                if training:
-                    ls = loss_streams[i]
-                    ls.wait_stream(dec_s)
-                    with torch.cuda.stream(ls):
-                        loss_ctxs.append(self.loss_fn.forward(y_true, cums, prepared))
-                        self._mark(f"fwd loss{i} done (side)")
-        main.wait_stream(dec_s)
-        main.wait_stream(aux[2])
-        if training:
-            main.wait_stream(side)
-            for ls in loss_streams:
-                main.wait_stream(ls)
-        self._mark("fwd joined (main)")
-        return cums, {"blocks": blocks, "loss": loss_ctxs, "y_true": y_true}
+        return {"main": main, "side": side, "aux": aux, "dec_s": aux[3], "x": x, "training": training, "use_dropout": use_dropout,
+                "seed_dev": seed_dev, "prepared": prepared, "loss_streams": loss_streams, "blocks": [], "loss_ctxs": []}
+
+    def _layer_block(self, st, i, x, cums):
+        """Boosted block i of the layer-level path on x [k, R, Cc, D] (any k).  Returns (encoder output, running
+        predictions), final on the dec stream."""
+        training, use_dropout, seed_dev = st["training"], st["use_dropout"], st["seed_dev"]
+        main, aux, dec_s = st["main"], st["aux"], st["dec_s"]
+        keys = self._keys(i) if use_dropout else None
+        enc = self.EncoderTransformerBlocks[i]
+        for blk in enc.EncoderBlocks:
+            blk.SelfAttentionBlock.rate = blk.FeedForwardBlock.rate = 0.1 if use_dropout else 0.0
+        dec_l = self.DecoderBlocks[i]
+        for nm in ("SelfAttentionBlock", "JointAttentionBlock", "FeedForwardBlock"):
+            if hasattr(dec_l, nm):
+                getattr(dec_l, nm).rate = 0.1 if use_dropout else 0.0
+        dkeys = keys["dec"] if keys else (0, 0, 0)
+        pre_self, dec0 = None, None
+        # (not on the very first call: layers build lazily in execution order, and the weight-initialisation
+        # order -- hence the seeded initial weights -- must not depend on this scheduling choice)
+        if hasattr(dec_l, "SelfAttentionBlock") and dec_l.SelfAttentionBlock.built:
+            aux[2].wait_stream(main)
+            with torch.cuda.stream(aux[2]):
+                dec0 = self.DecoderPrep.tile_queries(x.shape[0], like=x)
+                pre_self = dec_l.SelfAttentionBlock.forward([dec0, dec0, dec0], training, dkeys[0], seed_dev)
+        (x, pos), c_enc = enc.forward([x], training, keys["enc"] if keys else None, seed_dev)
+        self._mark(f"fwd enc{i} done (main)")
+        dec_s.wait_stream(main)
+        with torch.cuda.stream(dec_s):
+            prep_out, c_prep = self.DecoderPrep.forward([x, pos], training, dec=dec0)
+            if pre_self is not None:
+                dec_s.wait_stream(aux[2])
+            dec, c_dec = dec_l.forward(list(prep_out), training, dkeys, pre_self=pre_self, seed_dev=seed_dev)
+            self._mark(f"fwd dec{i} done (dec)")
+            mult = 2.0 if i == 0 else 1.0                 # block 0 is counted twice (reference :222-229)
+            if cums is not None and training:
+                cums = [c.clone() for c in cums]          # each block's loss keeps its own running prediction
+            heads = (self.CategoryBlocks[i], self.AttributeBlocks[i], self.BoxBlocks[i])
+            c_heads, new_cums = [], []
+            for h, head in enumerate(heads):              # three independent chains: one stream each
+                st_h = dec_s if h == 0 else aux[h - 1]
+                if st_h is not dec_s:
+                    st_h.wait_stream(dec_s)
+                with torch.cuda.stream(st_h):
+                    _, c = head.forward([dec], training, cum=None if cums is None else cums[h], mult=mult)
+                c_heads.append(c)
+                new_cums.append(c["cum"])
+            dec_s.wait_stream(aux[0])
+            dec_s.wait_stream(aux[1])
+            self._mark(f"fwd heads{i} done (dec)")
+            st["blocks"].append({"enc": c_enc, "prep": c_prep, "dec": c_dec, "heads": c_heads})
+        return x, new_cums
 
     def backward(self, ctx, gscale=1.0):
         """Gradient of gscale * sum_b sum_i total_b^(i) w.r.t. every trainable weight (accumulated).

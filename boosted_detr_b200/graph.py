@@ -185,8 +185,14 @@ class GraphedInference:
                 so the blocks after the exit block do not run (include/bdetr.h "Graph-captured inference").  The threshold
                 and `early_exit_min_blocks` live in device words: a change takes effect at the next call, without a new
                 capture.  Switching between None and a number needs a new GraphedInference.
-    `last_exit_block` and `last_image_confidence` are read from the device on first access after a call and equal what
-    the eager call leaves on the model (`last_image_confidence` is None when no block boundary was checked)."""
+      a number, with `model.early_exit_per_image` (and N >= 2): the per-image exit, captured as
+                    S0 -> SWITCH(h0){S1@k_min .. S1@B} -> ... -> SWITCH(h_{N-2}){S_{N-1}@k_min .. S_{N-1}@B}
+                where Si@k is block i at batch k plus boundary i's plan and compaction (the final write-out in block
+                N - 1); the plan of boundary i picks the body of block i + 1 that matches the images still running.
+                Changing `early_exit_per_image` after the capture needs a new GraphedInference.
+    `last_exit_block` and `last_image_confidence` (and in the per-image mode `last_exit_blocks` and `last_active_counts`)
+    are read from the device on first access after a call and equal what the eager call leaves on the model
+    (`last_image_confidence` is None when no block boundary was checked by the per-batch exit)."""
 
     def __init__(self, model, example_inputs, warmup=2):
         self.model = model
@@ -199,9 +205,11 @@ class GraphedInference:
         self.static_in = torch.empty(self.shape, dtype=torch.float32, device=require_cuda())
         self.segmented = model.early_exit_threshold is not None
         N, B, Q = model.num_decoder_blocks, self.shape[0], model.num_object_preds
+        self.per_image_flag = bool(model.early_exit_per_image)
+        self.per_image = self.segmented and self.per_image_flag and N >= 2
         self.load(example_inputs)
         self._exit_graph = None
-        if self.segmented:
+        if self.segmented and not self.per_image:
             # device words the decide kernels read: threshold (float32), min_blocks, threshold set; the exit block; the
             # image confidences of every boundary
             self._thr_dev = torch.zeros(1, dtype=torch.float32, device=require_cuda())
@@ -220,7 +228,17 @@ class GraphedInference:
             with torch.cuda.stream(side):
                 for _ in range(warmup):
                     cums = self._forward()[0]
-                if self.segmented:                 # load the decide / select kernels outside the capture
+                if self.per_image:                 # every kernel of every body size runs once outside the capture
+                    # with a threshold no image reaches, boundary 0 keeps all B slots in order, so block 1 may run at
+                    # any k <= B (its plan reads the first k slots of boundary 0's order)
+                    model.early_exit_threshold = 2.0
+                    st = model._per_image_begin(model._prepare({self.key: self.static_in}, False)[0])
+                    model._per_image_block(st, 0, B)
+                    for k in range(st["k_min"], B + 1):
+                        model._per_image_block(st, 1, k)
+                    self.k_min = st["k_min"]
+                    del st
+                elif self.segmented:               # load the decide / select kernels outside the capture
                     self._cums = [cums] * N
                     if N > 1:
                         self._decide(0, cums, 0)
@@ -229,7 +247,9 @@ class GraphedInference:
             torch.cuda.synchronize()
             model.early_exit_threshold = saved_thr
             t0 = time.perf_counter()
-            if self.segmented:
+            if self.per_image:
+                self._capture_switch()
+            elif self.segmented:
                 self._capture_segments()
             else:
                 self.graph = torch.cuda.CUDAGraph(keep_graph=True)
@@ -238,7 +258,8 @@ class GraphedInference:
             t1 = time.perf_counter()
             if self.segmented:
                 segs = (ctypes.c_void_p * len(self._segs))(*[g.raw_cuda_graph() for g in self._segs])
-                _lib.check(lib.bdetr_exit_graph_build(self._exit_graph, segs, len(self._segs)))
+                build = lib.bdetr_switch_graph_build if self.per_image else lib.bdetr_exit_graph_build
+                _lib.check(build(self._exit_graph, segs, len(self._segs)))
             else:
                 self.graph.instantiate()
             torch.cuda.synchronize()
@@ -279,6 +300,36 @@ class GraphedInference:
             self._begin_segment()
             self._select()
             self._segs[-1].capture_end()
+
+    def _capture_switch(self):
+        """S0 = prologue + block 0 + boundary 0, then block i at every batch k_min .. B, one body each, into one pool:
+        bodies of one SWITCH never run together and SWITCH i ends before SWITCH i + 1 begins, so memory a body frees
+        may serve the bodies captured after it.  What later bodies read (the gather buffers, outputs, plan state,
+        positional tables, hoisted self-attention) lives in the prologue's state, kept until close()."""
+        m = self.model
+        lib = _lib.load()
+        N, B = m.num_decoder_blocks, self.shape[0]
+        self._pool = torch.cuda.graph_pool_handle()
+        self._origin = torch.cuda.Stream()
+        self._origin.wait_stream(torch.cuda.current_stream())
+        self._segs = []
+        handles = (ctypes.c_ulonglong * (N - 1))()
+        g = ctypes.c_void_p()
+        _lib.check(lib.bdetr_switch_graph_create(N - 1, B - self.k_min + 1, ctypes.byref(g), handles))
+        self._exit_graph, self._handles = g, list(handles)
+        with torch.cuda.stream(self._origin):
+            self._begin_segment()
+            feats, _ = m._prepare({self.key: self.static_in}, False)
+            st = m._per_image_begin(feats)
+            m._per_image_block(st, 0, B, self._handles[0])
+            self._segs[-1].capture_end()
+            for i in range(1, N):
+                for k in range(self.k_min, B + 1):
+                    self._begin_segment()
+                    m._per_image_block(st, i, k, self._handles[i] if i < N - 1 else 0)
+                    self._segs[-1].capture_end()
+        self.out, self._keep = st["out"], (feats, st)
+        self.bodies = len(self._segs)
 
     def _begin_segment(self):
         g = torch.cuda.CUDAGraph(keep_graph=True)
@@ -347,6 +398,9 @@ class GraphedInference:
         if (m.early_exit_threshold is not None) != self.segmented:
             raise RuntimeError("early_exit_threshold changed between None and a number since the capture: the early exit "
                                "needs a differently shaped graph, capture a new GraphedInference")
+        if bool(m.early_exit_per_image) != self.per_image_flag:
+            raise RuntimeError("early_exit_per_image changed since the capture: the per-image exit needs a differently "
+                               "shaped graph, capture a new GraphedInference")
 
     def load(self, inputs):
         """Host or device input -> the static input buffer, async on the current stream."""
@@ -363,7 +417,10 @@ class GraphedInference:
             m._h2d(self.key, x, "f32", dst=dst)
 
     def replay(self):
-        if self.segmented:
+        if self.per_image:
+            self.model._exit_words()
+            _lib.check(_lib.load().bdetr_exit_graph_launch(self._exit_graph, stream_ptr()))
+        elif self.segmented:
             self._push_words()
             _lib.check(_lib.load().bdetr_exit_graph_launch(self._exit_graph, stream_ptr()))
         else:
@@ -387,7 +444,12 @@ class GraphedInference:
         if self._read is None:
             m = self.model
             N = m.num_decoder_blocks
-            if not self.segmented:
+            if self.per_image:
+                B = self.shape[0]
+                h = self._keep[1]["state"][:1 + N + 2 * B].cpu()
+                exits = h[1 + N:1 + N + B]
+                self._read = (int(exits.max()), h[1 + N + B:].view(torch.float32), exits, h[1:1 + N])
+            elif not self.segmented:
                 self._read = (N - 1, None)
             else:
                 e = int(self._exit_dev.item())
@@ -404,6 +466,14 @@ class GraphedInference:
     @property
     def last_image_confidence(self):
         return self._exit_state()[1]
+
+    @property
+    def last_exit_blocks(self):
+        return self._exit_state()[2] if self.per_image else None
+
+    @property
+    def last_active_counts(self):
+        return self._exit_state()[3] if self.per_image else None
 
     def close(self):
         if self._exit_graph is not None:

@@ -47,7 +47,8 @@ typedef enum {
 
 /* 101: attention at head dim 64 (D/H = 64) besides 32
  * 103: graph-captured inference with the early exit on the device (bdetr_exit_graph_*, bdetr_early_exit_decide)
- * 104: the attention core backward exported on its own (bdetr_attention_core_bwd) */
+ * 104: the attention core backward exported on its own (bdetr_attention_core_bwd)
+ * 105: per-image early exit: images leave the batch at their own boundary (bdetr_image_exit_*, bdetr_switch_graph_*) */
 int bdetr_version(void);
 const char *bdetr_last_error(void);
 /* Process-wide compute mode used by the dense entry points. */
@@ -544,6 +545,47 @@ int bdetr_early_exit_decide(int B, int boundary, int n_blocks, const float *imag
  * copies those of block *exit_block (read on the device) into cat / attr / box.  n_blocks <= BDETR_MAX_EXIT_BLOCKS. */
 int bdetr_select_exit_predictions(int n_blocks, int B, int Q, int C, int A, const float *const *cums,
                                   const int32_t *exit_block, float *cat, float *attr, float *box, void *stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Per-image early exit (inference).  Each image leaves the forward after its own boundary; the images still running are
+ * gathered to the front of the batch in order and the next block runs at that smaller batch k.  On a path whose GEMMs need
+ * k_min rows' worth of images (the fused tensor-core path: k_min = max(ceil(128 / L), ceil(128 / Q))) the batch never
+ * drops below k_min: images that have already left ride along (recomputed, never written again).
+ *   state   int32 words, bdetr_image_exit_state_bytes(B, N) bytes, allocated by the caller; nothing needs initialising.
+ *           word 0 n_active (images running the next block, riders included), 1 .. N counts[N] (images that ran each block),
+ *           then exit_block[B] (int32), conf[B] (float32: the image's confidence at its exit boundary, or at the last
+ *           boundary checked; NaN if none was), then private words (the slot order, the gather list, per-slot flags).
+ *   after block i < N - 1, on the block's stream:
+ *     bdetr_inverse_tokenize(k_in, ...) of the k_in running slots' category prediction, conf_scale = 1 / (i + 2);
+ *     bdetr_image_exit_plan(.., boundary i, k_in, image_conf, threshold, min_blocks, threshold_set, switch handle | 0, state):
+ *       one CTA; image_conf [k_in] in slot order; device words as for bdetr_early_exit_decide.  A live image leaves when
+ *       threshold_set, i + 1 >= min_blocks and image_conf >= threshold (float32, a NaN is not confident).  Writes the
+ *       new slot order and n_active = 0 if nobody stays, else max(stayers, k_min).  With a handle, sets it to
+ *       n_active - k_min, or B - k_min + 1 (no body) when nobody stays.  k_in == B at boundary 0.
+ *     bdetr_image_exit_compact(.., boundary i, k_in, ..): the running predictions cum_in [3] ([k_in, Q, C | A | 4]) of the
+ *       images leaving here -> out [3] ([B, Q, .]) at their original index; x_in [k_in, x_row] and cum_in of the next
+ *       block's slots -> x_out / cum_out (separate buffers of B rows; n_active rows are written, read on the device).
+ *   after block N - 1: bdetr_image_exit_compact(.., boundary N - 1, ..) writes every live slot's predictions to out
+ *     (x_in, x_out, cum_out may be NULL).  Needs n_blocks >= 2.
+ * ---------------------------------------------------------------------------------------- */
+size_t bdetr_image_exit_state_bytes(int B, int n_blocks);
+int bdetr_image_exit_plan(int B, int n_blocks, int k_min, int boundary, int k_in, const float *image_conf,
+                          const float *threshold, const int32_t *min_blocks, const int32_t *threshold_set,
+                          unsigned long long next_switch, int32_t *state, void *stream);
+int bdetr_image_exit_compact(int B, int n_blocks, int boundary, int k_in, int Q, int C, int A, long long x_row,
+                             const float *x_in, const float *const *cum_in, float *x_out, float *const *cum_out,
+                             float *const *out, const int32_t *state, void *stream);
+/* Graph of the per-image exit (SWITCH nodes, CUDA 12.8 driver or newer, else BDETR_E_UNSUPPORTED):
+ *   bdetr_switch_graph_create(N - 1, n_branches = B - k_min + 1, &g, handles): one SWITCH handle per boundary, default
+ *     value n_branches (matches no body: a SWITCH whose plan did not run launches nothing);
+ *   capture S0 = everything before block 0 + block 0 + boundary 0's plan (handle 0) and compaction, and for every
+ *     boundary i = 0 .. N - 2 and k = k_min .. B the body S_{i+1}@k = block i + 1 at batch k + boundary i + 1's plan
+ *     (handle i + 1) and compaction, or the final compaction in block N - 1;
+ *   bdetr_switch_graph_build(g, {S0, S1@k_min .. S1@B, S2@k_min, ...}, 1 + (N - 1) * n_branches)
+ *     -> child(S0) -> SWITCH(h0){S1@k_min .. S1@B} -> ... -> SWITCH(h_{N-2}){S_{N-1}@k_min .. S_{N-1}@B};
+ *   bdetr_exit_graph_launch / bdetr_exit_graph_destroy as above. */
+int bdetr_switch_graph_create(int n_boundaries, int n_branches, bdetr_exit_graph **g, unsigned long long *handles);
+int bdetr_switch_graph_build(bdetr_exit_graph *g, void *const *segments, int n_segments);
 
 /* ------------------------------------------------------------------------------------------
  * Data parallel (SURVEY 8e): the gradient all-reduce, the only collective on the path.  The reference's
